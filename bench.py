@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — image-pairs/sec of the newUNetTrans bitemporal forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload levir256|xbd1024]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--workload levir256|xbd1024] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +23,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (which may be read-only)
 
 import torch  # noqa: E402
 
@@ -231,6 +232,32 @@ def _time_steps(fn, steps, barrier):
     return e0.elapsed_time(e1)
 
 
+DUMP_BYTES = 64 * 10**6     # --dump-outputs: all files together
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (B, C, H, W) tensor as out_dir/<name>.npy in float32.  When the whole set would exceed DUMP_BYTES, each array
+    is reduced to its C values at a seeded sample of its (b, y, x) positions: <name>.npy is then (n, C) and <name>_index.npy
+    (n, 3) holds those positions (float32, exact).  The sample is the same for every run with the same arguments, so two runs or
+    two builds write files that compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    headers = 2 * 4096 * len(arrays)
+    if sum(t.numel() for t in arrays.values()) * 4 + headers <= DUMP_BYTES:
+        for name, t in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+        return
+    full = sum(t.numel() // t.shape[1] * (t.shape[1] + 3) * 4 for t in arrays.values())     # every position, values + index
+    for name, t in arrays.items():
+        B, C, H, W = t.shape
+        n = B * H * W * (DUMP_BYTES - headers) // full
+        pos = torch.randperm(B * H * W, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        x = t.detach().float().permute(0, 2, 3, 1).reshape(-1, C).cpu()[pos]
+        idx = torch.stack([pos // (H * W), pos // W % H, pos % W], 1).float()
+        np.save(os.path.join(out_dir, name + ".npy"), x.numpy())
+        np.save(os.path.join(out_dir, name + "_index.npy"), idx.numpy())
+
+
 def _training_leg(dev, batch=8, steps=10):
     import contextlib
     import torch.nn.functional as F
@@ -308,6 +335,13 @@ def run_native(a, wl):
     def step(i):
         return fwd(*sets[i % nsets])
 
+    last = {}
+
+    def timed_step(i):
+        y = step(i)
+        if i == a.steps - 1:
+            last["logits"] = y
+
     def barrier():
         if world > 1:
             dist.barrier()
@@ -320,7 +354,7 @@ def run_native(a, wl):
         sampler = ClockSampler(dev) if rank == 0 else None
         if sampler:
             sampler.start()
-        ms = _time_steps(step, a.steps, barrier)
+        ms = _time_steps(timed_step, a.steps, barrier)
         # ---- strong scaling (configs[1] as written: ONE global batch of 64 pairs split 64/N per rank, no collective)
         gB = wl["pairs"]
         sB = max(1, gB // world)
@@ -568,6 +602,8 @@ def run_native(a, wl):
                 roofline=roof, top_kernels=[dict(name=k["name"], ms=round(k["ms"], 4)) for k in kernels])
     if cpu:
         line["cpu_baseline"] = cpu
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, last)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -589,7 +625,15 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity block (oracle on CPU + other modes)")
     ap.add_argument("--ref-pairs", type=int, default=None, help="--impl reference: pairs per step (default: the workload batch for LEVIR, 1 for xBD)")
     ap.add_argument("--dump-kernels", default=None, help="write the per-launch table (name, ms, flops, bytes) to this JSON file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (rank 0) to DIR/<name>.npy in float32, at most 64 MB in all "
+                         "(beyond that, the values at a fixed seeded sample of (b, y, x) positions, listed in DIR/<name>_index.npy); "
+                         "the inputs depend only on the arguments")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the native arm's outputs; the reference arm times other inputs (one CPU sample)")
     wl = WORKLOADS[a.workload]
     if a.impl == "reference":
         return run_reference(a, wl)

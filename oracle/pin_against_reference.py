@@ -155,13 +155,13 @@ def main():
         assert d <= 4 * noise + 1e-6, name
         report[name] = dict(semantic_fp64=sem, fp32_oracle_vs_ref=d, ref_fp32_noise=noise, argmax_agree=agree,
                             logit_std=float(y_ref.std()))
-        np.savez_compressed(os.path.join(GOLD, name + ".npz"),
-                            logits=y_ref.numpy().astype(np.float32),
-                            logits_f64ref=y_ref64.numpy().astype(np.float32),
-                            tokens_5=taps_ref["tokens_5"].numpy(), tokens_4=taps_ref["tokens_4"].numpy(),
-                            tokens_3=taps_ref["tokens_3"].numpy(),
-                            level_5=taps["level_5"].numpy().astype(np.float32),
-                            level_4=taps["level_4"].numpy().astype(np.float32))
+        # what the tests read, nothing more (every fixture stays under 1 MB): the fp32 reference logits are skipped where the
+        # fp32 reference is itself 1e-4 away from its fp64 self (levir_synth3_uniform); the tests compare with the fp64 one there
+        fix = dict(logits_f64ref=y_ref64.numpy().astype(np.float32),
+                   tokens_5=taps_ref["tokens_5"].numpy(), tokens_4=taps_ref["tokens_4"].numpy(), tokens_3=taps_ref["tokens_3"].numpy())
+        if name != "levir_synth3_uniform":
+            fix["logits"] = y_ref.numpy().astype(np.float32)
+        np.savez_compressed(os.path.join(GOLD, name + ".npz"), **fix)
     del ref64
     # (d) xBD variant, 1024x1024, B=1, 5 classes (subsampled fixture: every 8th pixel + float64 checksums)
     sxs = synth.synth_state_dict(sxr, seed=6, style="default")

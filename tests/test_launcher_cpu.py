@@ -1,5 +1,6 @@
-"""CPU: the launcher swaps the class inside the UNMODIFIED reference's define_G (build container only — needs
-/root/reference), and the world_size-2 gloo path of the pair sharding used by bench.py."""
+"""CPU: the launcher swaps the class inside the UNMODIFIED reference's define_G (needs the original DAHiTra sources:
+$DAHITRA_REFERENCE, else the copy baseline/install_reference.py places under baseline/_ref/ref), and the world_size-2
+gloo path of the pair sharding used by bench.py."""
 import os
 import subprocess
 import sys
@@ -7,10 +8,11 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("DAHITRA_REFERENCE", os.path.join(ROOT, "baseline", "_ref", "ref"))
+NO_REF = f"original DAHiTra sources not found at {REF} (set DAHITRA_REFERENCE or run baseline/install_reference.py)"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason=NO_REF)
 def test_reference_define_G_builds_the_native_class():
     code = (
         "import torch\n"
@@ -28,7 +30,7 @@ def test_reference_define_G_builds_the_native_class():
     assert "OK" in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason=NO_REF)
 def test_pretrained_trunk_path_equals_the_reference(tmp_path):
     """The reference's define_G with its pretrained=True trunk left ON (models/networks.py:1096; load_state_dict_from_url served
     from a local file instead of the network) against dahitra_b200's define_G reading the same file: all 425 tensors bit-identical

@@ -1,5 +1,6 @@
 """Device-side confusion matrix / scores (SURVEY.md §8 f1) against the numpy restatement of misc/metric_tool.py,
-which is itself pinned against the reference module when /root/reference is present."""
+which is itself pinned against the reference module when the original DAHiTra sources are present ($DAHITRA_REFERENCE,
+else the copy baseline/install_reference.py places under baseline/_ref/ref)."""
 import importlib.util
 import os
 
@@ -9,7 +10,9 @@ import torch
 
 from oracle import metrics_oracle as MO
 
-REF = "/root/reference/misc/metric_tool.py"
+REF_DIR = os.environ.get("DAHITRA_REFERENCE", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                                                           "baseline", "_ref", "ref"))
+REF = os.path.join(REF_DIR, "misc", "metric_tool.py")
 
 
 def _maps(seed, n, nc, ignore=True):
@@ -21,7 +24,8 @@ def _maps(seed, n, nc, ignore=True):
     return pr, gt
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not os.path.exists(REF), reason=f"original DAHiTra sources not found: {REF} "
+                                                   "(set DAHITRA_REFERENCE or run baseline/install_reference.py)")
 def test_oracle_matches_reference_metric_tool():
     spec = importlib.util.spec_from_file_location("ref_metric_tool", REF)
     ref = importlib.util.module_from_spec(spec)

@@ -16,7 +16,7 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref", "ref")
+REF = os.environ.get("DAHITRA_REFERENCE", os.path.join(ROOT, "baseline", "_ref", "ref"))
 have_ref = os.path.exists(os.path.join(REF, "models", "evaluator.py")) and os.path.isdir(os.path.join(REF, "data", "LEVIR_CD", "train", "A"))
 
 
@@ -28,7 +28,8 @@ def run_harness(impl, device, what="eval,train"):
     return json.loads(line.split("HARNESS_JSON ", 1)[1])
 
 
-@pytest.mark.skipif(not have_ref, reason="baseline/_ref/ref not installed (python baseline/install_reference.py)")
+@pytest.mark.skipif(not have_ref, reason=f"original DAHiTra sources and LEVIR samples not found at {REF} "
+                                         "(set DAHITRA_REFERENCE or run baseline/install_reference.py)")
 def test_reference_evaluator_on_reference_class_equals_oracle_cpu():
     out = run_harness("reference", "cpu", what="eval")
     assert out["eval_net_class"] == "models.networks"
@@ -40,7 +41,8 @@ def test_reference_evaluator_on_reference_class_equals_oracle_cpu():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not have_ref, reason="baseline/_ref/ref not installed (python baseline/install_reference.py)")
+@pytest.mark.skipif(not have_ref, reason=f"original DAHiTra sources and LEVIR samples not found at {REF} "
+                                         "(set DAHITRA_REFERENCE or run baseline/install_reference.py)")
 def test_unmodified_evaluator_and_trainer_on_native_module():
     out = run_harness("native", "cuda")
     print("[harness]", {k: out[k] for k in ("eval_net_class", "eval_cm", "oracle_cm", "logits_max_abs_diff_vs_oracle",
