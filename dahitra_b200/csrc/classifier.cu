@@ -12,6 +12,9 @@
 //     on one half, a producer warp has the next one in flight (full / empty mbarriers).
 // CTA tile = 32 x 16 pixels; thread (lx, g) owns the 4 vertically adjacent pixels (lx, 4g..4g+3), so each 128-bit halo
 // read feeds up to 3 output rows and each filter read feeds 4 pixels.
+// H16: the input is one FP16 plane (the h16 mode).  A 64-byte row then holds all 32 channels of a pixel, so one box
+// {32 ch, 40, 18, 1} per tile (the same bytes and swizzle as one fp32 half); every 16-byte read is converted to eight
+// fp32 values and summed with the same packed FFMA2 / scalar chains.
 #include "tc_common.cuh"
 #include <cstdlib>
 
@@ -27,11 +30,13 @@ constexpr uint32_t CT_BUF = CT_HALF_BYTES;
 constexpr int CT_NBUF = 2;
 constexpr int CT_THREADS = 160;                                      // 4 compute warps + 1 producer warp
 
-template <int NC>
+template <int NC, bool H16>
 __global__ void __launch_bounds__(CT_THREADS, 2)
 classifier_tma_kernel(const __grid_constant__ CUtensorMap tmIn, int H, int W, int tilesX, int tilesY, int ntiles,
                       const float* __restrict__ w, const float* __restrict__ bias, float* __restrict__ logits,
                       unsigned char* __restrict__ amax) {
+  constexpr int NPASS = H16 ? 1 : 2;                                  // boxes per tile
+  constexpr int PCH = H16 ? 32 : CT_CH;                               // channels per box
   extern __shared__ uint8_t ct_raw[];
   __shared__ __align__(8) uint64_t full[CT_NBUF], empty[CT_NBUF];
   const uint32_t base = (smem_u32(ct_raw) + 1023u) & ~1023u;
@@ -54,7 +59,7 @@ classifier_tma_kernel(const __grid_constant__ CUtensorMap tmIn, int H, int W, in
       for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         const int tx = tile % tilesX, ty = (tile / tilesX) % tilesY, n = tile / (tilesX * tilesY);
 #pragma unroll
-        for (int pass = 0; pass < 2; ++pass, ++q) {
+        for (int pass = 0; pass < NPASS; ++pass, ++q) {
           const int b = q % CT_NBUF;
           mbar_wait(smem_u32(&empty[b]), (uint32_t)(((q / CT_NBUF) & 1) ^ 1));
           mbar_expect_tx(smem_u32(&full[b]), CT_HALF_BYTES);
@@ -91,24 +96,34 @@ classifier_tma_kernel(const __grid_constant__ CUtensorMap tmIn, int H, int W, in
         if (PACK) acc2[j][k] = make_float2(bsv[k], 0.f);
       }
 #pragma unroll 1
-    for (int pass = 0; pass < 2; ++pass, ++q) {
+    for (int pass = 0; pass < NPASS; ++pass, ++q) {
       const int b = q % CT_NBUF;
       mbar_wait(smem_u32(&full[b]), (uint32_t)((q / CT_NBUF) & 1));
       const float* halo = reinterpret_cast<const float*>(bp + (size_t)b * CT_BUF);     // [18 x 40 pixels][16 ch], 64-byte rows, SWIZZLE_64B
 #pragma unroll
       for (int s = 0; s < 3; ++s) {
-#pragma unroll
-        for (int c4 = 0; c4 < CT_CH / 4; ++c4) {
+        // H16 at 7 / 8 classes: the full unroll spills (8 classes still spill 12 bytes at the 168-register cap of two CTAs per
+        // SM, like the fp32 form); the network runs 2 and 5 classes
+        constexpr int C4_UNROLL = (H16 && NC >= 7) ? 2 : 8;
+#pragma unroll C4_UNROLL
+        for (int c4 = 0; c4 < (H16 ? 8 : CT_CH / 4); ++c4) {     // 4-channel groups (H16: two per 16-byte chunk)
           float4 ww[3][NC];                                // the three filter rows of column s for these 4 channels
 #pragma unroll
           for (int r = 0; r < 3; ++r)
 #pragma unroll
             for (int k = 0; k < NC; ++k)
-              ww[r][k] = *reinterpret_cast<const float4*>(&w_s[((r * 3 + s) * NC + k) * 32 + pass * CT_CH + c4 * 4]);
+              ww[r][k] = *reinterpret_cast<const float4*>(&w_s[((r * 3 + s) * NC + k) * 32 + pass * PCH + c4 * 4]);
 #pragma unroll
           for (int hr = 0; hr < 6; ++hr) {                 // halo row 4g + hr feeds output rows j = hr - r, r = 0..2
             // halo pixel p = (4g + hr) * 40 + lx + s; SWIZZLE_64B puts its chunk c4 at c4 ^ ((p >> 1) & 3) = c4 ^ (((lx + s) >> 1) & 3)
-            const float4 v = *reinterpret_cast<const float4*>(&halo[(4 * g + hr) * (CT_HW * CT_CH) + choff[s][c4]]);
+            float4 v;
+            if (H16) {                                     // the 16-byte chunk c4 / 2 holds 8 channels; this group is its half c4 & 1
+              const int ch = (lx + s) * CT_CH + (((c4 >> 1) ^ (((lx + s) >> 1) & 3)) << 2);   // = choff[s][c4 >> 1]
+              const uint2 u = reinterpret_cast<const uint2*>(&halo[(4 * g + hr) * (CT_HW * CT_CH) + ch])[c4 & 1];
+              v = make_float4(f16_lo(u.x), f16_hi(u.x), f16_lo(u.y), f16_hi(u.y));
+            } else {
+              v = *reinterpret_cast<const float4*>(&halo[(4 * g + hr) * (CT_HW * CT_CH) + choff[s][c4]]);
+            }
 #pragma unroll
             for (int r = 0; r < 3; ++r) {
               const int j = hr - r;
@@ -158,8 +173,10 @@ classifier_tma_kernel(const __grid_constant__ CUtensorMap tmIn, int H, int W, in
 }
 }  // namespace
 
-int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const float* w, const float* b,
-                             float* logits, unsigned char* amax, cudaStream_t s) {
+namespace {
+template <bool H16>
+int launch_classifier(const void* in, int N, int H, int W, int nc, const float* w, const float* b, float* logits,
+                      unsigned char* amax, cudaStream_t s) {
   DH_REQUIRE(in && w && b && logits, DH_E_NULL);
   DH_REQUIRE(N > 0 && H > 0 && W > 0 && nc >= 1 && nc <= 8, DH_E_SHAPE);
   DH_REQUIRE(dh_aligned16(in) && dh_aligned16(w), DH_E_ALIGN);
@@ -167,10 +184,11 @@ int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const
   const int ntiles = tx * ty * N;
   CUtensorMap tm;
   {
+    const unsigned long long eb = H16 ? 2ull : 4ull;                   // bytes per element
     const unsigned long long dims[4] = {32ull, (unsigned long long)W, (unsigned long long)H, (unsigned long long)N};
-    const unsigned long long strides[3] = {128ull, (unsigned long long)W * 128ull, (unsigned long long)H * W * 128ull};
-    const unsigned box[4] = {(unsigned)CT_CH, (unsigned)CT_HW, (unsigned)CT_HH, 1u};
-    const int rc = dh_encode_tiled_f32_sw(&tm, in, 4, dims, strides, box, 64);
+    const unsigned long long strides[3] = {32 * eb, (unsigned long long)W * 32 * eb, (unsigned long long)H * W * 32 * eb};
+    const unsigned box[4] = {H16 ? 32u : (unsigned)CT_CH, (unsigned)CT_HW, (unsigned)CT_HH, 1u};
+    const int rc = H16 ? dh_encode_tiled_f16_sw(&tm, in, 4, dims, strides, box, 64) : dh_encode_tiled_f32_sw(&tm, in, 4, dims, strides, box, 64);
     if (rc) return rc;
   }
   int dev = 0, sms = 148;
@@ -180,9 +198,9 @@ int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const
 #define DH_CLS_CASE(NC)                                                                                                 \
   case NC: {                                                                                                            \
     const int smem = (int)(CT_NBUF * CT_BUF + 9 * NC * 32 * sizeof(float) + 1024);                                      \
-    cudaError_t e = cudaFuncSetAttribute(classifier_tma_kernel<NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); \
+    cudaError_t e = cudaFuncSetAttribute(classifier_tma_kernel<NC, H16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); \
     if (e != cudaSuccess) return (int)e;                                                                                \
-    return dh_launch(classifier_tma_kernel<NC>, grid, dim3(CT_THREADS), (size_t)smem, s, tm, H, W, tx, ty, ntiles, w, b, logits, amax); \
+    return dh_launch(classifier_tma_kernel<NC, H16>, grid, dim3(CT_THREADS), (size_t)smem, s, tm, H, W, tx, ty, ntiles, w, b, logits, amax); \
   }
   switch (nc) {
     DH_CLS_CASE(1) DH_CLS_CASE(2) DH_CLS_CASE(3) DH_CLS_CASE(4)
@@ -190,4 +208,14 @@ int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const
   }
 #undef DH_CLS_CASE
   return DH_E_SHAPE;
+}
+}  // namespace
+
+int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const float* w, const float* b,
+                             float* logits, unsigned char* amax, cudaStream_t s) {
+  return launch_classifier<false>(in, N, H, W, nc, w, b, logits, amax, s);
+}
+int dh_launch_classifier_h16(const void* in, int N, int H, int W, int nc, const float* w, const float* b,
+                             float* logits, unsigned char* amax, cudaStream_t s) {
+  return launch_classifier<true>(in, N, H, W, nc, w, b, logits, amax, s);
 }

@@ -69,11 +69,13 @@ struct Conv3Args {
   const float* bias; const void* res; int res_split; // residual: fp32 NHWC or split16 (same shape as the output)
   int relu;
   void* out; int out_split;                          // fp32 NHWC or split16
-  int ps = 0;                                        // pixel-shuffle store of a 32 -> 4x32 upsample convolution (fp32 output only)
+  int ps = 0;                                        // pixel-shuffle store of a 32 -> 4x32 upsample convolution (fp32 output, or h16)
   int tok = 0;                                       // tokenizer epilogue (1x1, Cout 32): ReLU + store + per-tile softmax partials
   const float* wtok = nullptr; float* partials = nullptr;
   int force_stream = 0;                              // 1: never keep the filter resident in shared memory (A/B tests)
   int cg = 0;                                        // 0 = auto, 1 = single CTAs, 2 = CTA pairs (tcgen05 cta_group::2)
+  int h16 = 0;                                       // 1: in0 / in1 and a split16 res / out are ONE FP16 plane each (in*_plane,
+                                                     // res_plane, out_plane unused), the filter contributes h_w alone; no CTA pairs
 };
 bool dh_conv_tc3_eligible(const Conv3Args& a);
 int dh_launch_conv_tc3(const Conv3Args& a, cudaStream_t s);
@@ -82,6 +84,7 @@ int dh_conv_tc3_tok_chunks(int H, int W);            // partial-softmax chunks p
 int dh_launch_split_pack(const float* in, size_t n, void* out, cudaStream_t s);
 int dh_launch_split_unpack(const void* in, size_t n, float* out, cudaStream_t s);
 int dh_launch_maxpool_split(const void* in, int N, int H, int W, int C, void* out, cudaStream_t s);
+int dh_launch_maxpool_h16(const void* in, int N, int H, int W, int C, void* out, cudaStream_t s);      // one FP16 plane
 // programmatic dependent launch: attribute for cudaLaunchKernelEx (returns the number of attributes written: 0 or 1)
 int dh_pdl_attr(cudaLaunchAttribute* at);
 void dh_set_pdl(int on);
@@ -114,6 +117,8 @@ int dh_launch_maxpool(const float* in, int N, int H, int W, int C, float* out, c
 int dh_launch_classifier(const float* in, int N, int H, int W, int nc, const float* w, const float* b,
                          float* logits, unsigned char* amax, cudaStream_t s);
 int dh_launch_classifier_tma(const float* in, int N, int H, int W, int nc, const float* w, const float* b,
+                             float* logits, unsigned char* amax, cudaStream_t s);
+int dh_launch_classifier_h16(const void* in, int N, int H, int W, int nc, const float* w, const float* b,    // one FP16 plane in
                              float* logits, unsigned char* amax, cudaStream_t s);
 int dh_launch_squeeze_tokens(const float* feat, int N, int npix, int Cin, const float* wsq, const float* wtok,
                              float* xs, float* partials, cudaStream_t s);

@@ -630,7 +630,7 @@ int dh_encode_tiled_f32(CUtensorMap* out, const void* ptr, int rank, const unsig
   return dh_encode_tiled_f32_sw(out, ptr, rank, dims, strides, box, swizzle128 ? 128 : 0);
 }
 // swizzle_bytes: 0 (none), 64 or 128
-int dh_encode_tiled_f32_sw(CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,
+static int encode_tiled_sw(CUtensorMapDataType dtype, CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,
                            const unsigned long long* strides, const unsigned* box, int swizzle_bytes) {
   EncodeTiledFn enc = get_encode2();
   if (!enc) return DH_E_VARIANT;
@@ -638,11 +638,19 @@ int dh_encode_tiled_f32_sw(CUtensorMap* out, const void* ptr, int rank, const un
   cuuint32_t b[5], es[5] = {1, 1, 1, 1, 1};
   for (int i = 0; i < rank; ++i) { d[i] = dims[i]; b[i] = box[i]; }
   for (int i = 0; i + 1 < rank; ++i) st[i] = strides[i];
-  const CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void*>(ptr), d, st, b, es,
+  const CUresult r = enc(out, dtype, (cuuint32_t)rank, const_cast<void*>(ptr), d, st, b, es,
                          CU_TENSOR_MAP_INTERLEAVE_NONE,
                          swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE),
                          CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? 0 : DH_E_SHAPE;
+}
+int dh_encode_tiled_f32_sw(CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,
+                           const unsigned long long* strides, const unsigned* box, int swizzle_bytes) {
+  return encode_tiled_sw(CU_TENSOR_MAP_DATA_TYPE_FLOAT32, out, ptr, rank, dims, strides, box, swizzle_bytes);
+}
+int dh_encode_tiled_f16_sw(CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,
+                           const unsigned long long* strides, const unsigned* box, int swizzle_bytes) {
+  return encode_tiled_sw(CU_TENSOR_MAP_DATA_TYPE_FLOAT16, out, ptr, rank, dims, strides, box, swizzle_bytes);
 }
 
 namespace {

@@ -24,7 +24,11 @@
 // loop — the epilogue-heavy shapes (tokenizer squeeze, pixel-shuffle convs, residual + split16 stores) were bound by one.
 //
 // Epilogue outputs: fp32 NHWC (optionally as the pixel-shuffle scatter of the upsample convolutions) or split16 planes;
-// the residual may be fp32 or split16.  TOK epilogue (1x1 squeeze convolution of the tokenizer, reference
+// the residual may be fp32 or split16.
+//
+// Single-plane form (P1, the h16 mode): activations are stored as ONE FP16 plane (hi alone, 2 bytes per element) and the
+// filter contributes h_w alone.  Per chunk one halo box, per (tap, chunk, K = 16 step) one N = NT MMA [h_a] x [h_w], an
+// accumulator of NT columns; the epilogue stores one FP16 plane (plain or pixel-shuffle) or fp32, and reads an FP16 residual.  TOK epilogue (1x1 squeeze convolution of the tokenizer, reference
 // models/networks.py:1177-1189, 1273-1280): ReLU, store, and the per-tile online-softmax partials (m, s, t[32]) of the four
 // semantic tokens — what squeeze_tokens_kernel (tokens.cu) computes on CUDA cores in the other modes.
 #include "tc_common.cuh"
@@ -59,16 +63,17 @@ struct T3Args {
 //              memory once per CTA and stays there while the persistent CTA walks its tiles — the L2 -> SM path
 //              (~43 B/clk per SM with every SM pulling, B300_MICROARCH "LTS throughput cap") is what bounds the
 //              streaming form on the small-K layers: layer1 re-reads 144 KB of filter for every 46 KB halo.
-template <int NT, bool RES, int CG = 1> struct T3Cfg {
+template <int NT, bool RES, int CG = 1, bool P1 = false> struct T3Cfg {
   static constexpr int TPS = NT == 128 ? 1 : 3;                          // filter taps per ring stage (streaming form)
   static constexpr int STAGES = RES ? 1 : (NT == 128 ? 6 : (NT == 64 ? 4 : 8)) * CG;   // a CTA of a pair holds half-size tiles
-  static constexpr uint32_t B_TAP = 2u * NT * 64u / CG;                  // [h_w ; l_w] x 64 B: NT rows each, NT / 2 in a CTA of a pair
+  static constexpr uint32_t HALO = P1 ? T3_PLANE : T3_HALO;             // bytes of one halo buffer
+  static constexpr uint32_t B_TAP = (P1 ? 1u : 2u) * NT * 64u / CG;      // [h_w ; l_w] (P1: h_w) x 64 B: NT rows each, NT / 2 in a CTA of a pair
   static constexpr uint32_t B_STAGE = B_TAP * TPS;
   static constexpr uint32_t RING_BYTES = RES ? 0u : STAGES * B_STAGE;    // RES: the filter image follows the halo buffers instead
   static constexpr int THREADS = 352;                                    // 11 warps: halo, MMA, epilogue A x4, filter, epilogue B x4
   static constexpr uint32_t IDESC_WIDE = umma_idesc_f16(128, 2 * NT);
   static constexpr uint32_t IDESC_NARROW = umma_idesc_f16(128 * CG, NT);
-  static constexpr int ACC_COLS = 2 * NT;
+  static constexpr int ACC_COLS = P1 ? NT : 2 * NT;
   static constexpr uint32_t TMEM_COLS = 2 * ACC_COLS < 32 ? 32 : 2 * ACC_COLS;
 };
 
@@ -126,6 +131,10 @@ __device__ __forceinline__ void join8(const uint4& hi, const uint4& lo, float4& 
   b = make_float4(fmaf(f16_lo(lo.z), S, f16_lo(hi.z)), fmaf(f16_hi(lo.z), S, f16_hi(hi.z)),
                   fmaf(f16_lo(lo.w), S, f16_lo(hi.w)), fmaf(f16_hi(lo.w), S, f16_hi(hi.w)));
 }
+__device__ __forceinline__ void half8(const uint4& h, float4& a, float4& b) {     // eight FP16 values -> fp32
+  a = make_float4(f16_lo(h.x), f16_hi(h.x), f16_lo(h.y), f16_hi(h.y));
+  b = make_float4(f16_lo(h.z), f16_hi(h.z), f16_lo(h.w), f16_hi(h.w));
+}
 __device__ __forceinline__ uint4 ldg16(const void* p) { return __ldg(reinterpret_cast<const uint4*>(p)); }
 __device__ __forceinline__ float4 as_f4(const uint4& u) { return make_float4(__uint_as_float(u.x), __uint_as_float(u.y), __uint_as_float(u.z), __uint_as_float(u.w)); }
 
@@ -136,12 +145,12 @@ __device__ __forceinline__ float4 as_f4(const uint4& u) { return make_float4(__u
 // three N = NT MMAs: h_a.h_w -> main; h_a.l_w, l_a.h_w -> corr — the same tensor-core cycles as wide + narrow.
 // Barriers the MMA warp waits on live in the leader and count both CTAs (the peer's TMA / threads signal them remotely);
 // the leader's commits are multicast to both CTAs' barriers.
-template <int NT, int KS, int SD, int EPI, bool RES, int CG>
-__global__ void __launch_bounds__(T3Cfg<NT, RES, CG>::THREADS, 1)
+template <int NT, int KS, int SD, int EPI, bool RES, int CG, bool P1>
+__global__ void __launch_bounds__(T3Cfg<NT, RES, CG, P1>::THREADS, 1)
 conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant__ CUtensorMap tmA0l,
                 const __grid_constant__ CUtensorMap tmA1h, const __grid_constant__ CUtensorMap tmA1l,
                 const __grid_constant__ CUtensorMap tmB, const T3Args e) {
-  using Cfg = T3Cfg<NT, RES, CG>;
+  using Cfg = T3Cfg<NT, RES, CG, P1>;
   constexpr int STAGES = Cfg::STAGES;
   extern __shared__ uint8_t t3_raw[];
   __shared__ __align__(8) uint64_t halo_full[T3_MAX_HB], halo_empty[T3_MAX_HB], b_full[STAGES], b_empty[STAGES], acc_full[2], acc_empty[2];
@@ -151,7 +160,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
   const uint32_t base = (smem_u32(t3_raw) + 1023u) & ~1023u;
   uint8_t* base_ptr = t3_raw + (base - smem_u32(t3_raw));
   const int HB = e.hb;
-  const uint32_t b_ring = base + (uint32_t)HB * T3_HALO;                 // filter ring, or the resident filter image
+  const uint32_t b_ring = base + (uint32_t)HB * Cfg::HALO;                 // filter ring, or the resident filter image
   const int rank = CG == 2 ? (int)cluster_ctarank() : 0;
   const int w0 = CG == 2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;      // first work item, and the stride between items
   const int wstep = CG == 2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
@@ -162,7 +171,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
   constexpr int TPS = (SD == 1 && NTAPS % Cfg::TPS == 0) ? Cfg::TPS : 1;
   constexpr int HALO_W = (KS == 3) ? T3_HW : T3_TW;
   const uint32_t w_bytes = RES ? (uint32_t)(e.ncout_tiles * e.cchunks * NTAPS) * Cfg::B_TAP : Cfg::RING_BYTES;
-  const uint32_t epi_off = (uint32_t)HB * T3_HALO + w_bytes;            // epilogue staging (8 warps x 4 KB), then the tok scratch
+  const uint32_t epi_off = (uint32_t)HB * Cfg::HALO + w_bytes;            // epilogue staging (8 warps x 4 KB), then the tok scratch
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < T3_MAX_HB; ++i) { mbar_init(smem_u32(&halo_full[i]), 1); mbar_init(smem_u32(&halo_empty[i]), 1); }
@@ -206,7 +215,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
   pdl_launch_dependents();
 
   if (warp == 0) {
-    if (lane == 0) {                                            // ---------------- halo TMA producer: hi + lo boxes per chunk
+    if (lane == 0) {                                            // ---------------- halo TMA producer: hi + lo boxes per chunk (P1: hi)
       int hb = 0;
       uint32_t ephase = 1;                                      // first pass over the ring: the buffers are free
       for (int tile = w0; tile < e.ntiles; tile += wstep) {
@@ -216,8 +225,8 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
           for (int ph = 0; ph < NPH; ++ph) {
             mbar_wait(smem_u32(&halo_empty[hb]), ephase);
             const uint32_t bar = smem_u32(&halo_full[hb]);
-            if (rank == 0) mbar_expect_tx(bar, (uint32_t)CG * 2u * e.halo_plane_bytes);     // pair: the leader's barrier counts both halos
-            const uint32_t dst = base + (uint32_t)hb * T3_HALO;
+            if (rank == 0) mbar_expect_tx(bar, (uint32_t)CG * (P1 ? 1u : 2u) * e.halo_plane_bytes);   // pair: the leader's barrier counts both halos
+            const uint32_t dst = base + (uint32_t)hb * Cfg::HALO;
             const int cx = SD == 1 ? t.ox0 - pad : 2 * (t.ox0 - pad) + (ph & 1);
             const int cy = SD == 1 ? t.oy0 - pad : 2 * (t.oy0 - pad) + (ph >> 1);
             const bool first = cc < e.cchunks0;
@@ -228,7 +237,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
               tma_load_4d_2sm(dst + T3_PLANE, first ? &tmA0l : &tmA1l, lbar, c0, cx, cy, t.n);
             } else {
               tma_load_4d(dst, first ? &tmA0h : &tmA1h, bar, c0, cx, cy, t.n);
-              tma_load_4d(dst + T3_PLANE, first ? &tmA0l : &tmA1l, bar, c0, cx, cy, t.n);
+              if (!P1) tma_load_4d(dst + T3_PLANE, first ? &tmA0l : &tmA1l, bar, c0, cx, cy, t.n);
             }
             if (++hb == HB) { hb = 0; ephase ^= 1u; }
           }
@@ -277,7 +286,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
           for (int ph = 0; ph < NPH; ++ph) {
             mbar_wait(smem_u32(&halo_full[hb]), hphase);
             tc_fence_after();
-            const uint32_t h_hi = base + (uint32_t)hb * T3_HALO, h_lo = h_hi + T3_PLANE;
+            const uint32_t h_hi = base + (uint32_t)hb * Cfg::HALO, h_lo = h_hi + T3_PLANE;
 #pragma unroll
             for (int i0 = Sched::first(ph); i0 < Sched::first(ph + 1); i0 += TPS) {
               uint32_t b_stage;
@@ -303,6 +312,9 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
                   for (int k = 0; k < 2; ++k) umma_bf16_2sm(d_corr, a_h + (uint64_t)(2 * k), b_l + (uint64_t)(2 * k), Cfg::IDESC_NARROW, (cc | i | k) ? 1u : 0u);
 #pragma unroll
                   for (int k = 0; k < 2; ++k) umma_bf16_2sm(d_corr, a_l + (uint64_t)(2 * k), b_w + (uint64_t)(2 * k), Cfg::IDESC_NARROW, 1u);
+                } else if (P1) {
+#pragma unroll
+                  for (int k = 0; k < 2; ++k) umma_bf16(d_main, a_h + (uint64_t)(2 * k), b_w + (uint64_t)(2 * k), Cfg::IDESC_NARROW, (cc | i | k) ? 1u : 0u);
                 } else {
 #pragma unroll
                   for (int k = 0; k < 2; ++k) umma_bf16(d_main, a_h + (uint64_t)(2 * k), b_w + (uint64_t)(2 * k), Cfg::IDESC_WIDE, (cc | i | k) ? 1u : 0u);
@@ -357,7 +369,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
           ra[g] = make_uint4(0u, 0u, 0u, 0u); rb[g] = ra[g];
           if (ok[g]) {
             const size_t o = rowoff[g] + (size_t)j * 32;
-            if (e.res_split) { ra[g] = ldg16(resb + o * 2); rb[g] = ldg16(resb + (o + (size_t)e.res_plane) * 2); }
+            if (e.res_split) { ra[g] = ldg16(resb + o * 2); if (!P1) rb[g] = ldg16(resb + (o + (size_t)e.res_plane) * 2); }
             else             { ra[g] = ldg16(resb + o * 4); rb[g] = ldg16(resb + o * 4 + 16); }
           }
         }
@@ -372,7 +384,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
         if (e.bias) { bia0 = ldg4(e.bias + n0 + j * 32 + c4 * 8); bia1 = ldg4(e.bias + n0 + j * 32 + c4 * 8 + 4); }
         uint32_t v[32], u[32];
         tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * Cfg::ACC_COLS + j * 32), v);
-        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * Cfg::ACC_COLS + NT + j * 32), u);
+        if (!P1) tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * Cfg::ACC_COLS + NT + j * 32), u);
         if (j == NSLAB - 1) {                                    // accumulator fully read: hand it back to the MMA warp
           tc_fence_before();
           if (CG == 2) mbar_arrive_cluster(mapa_u32(smem_u32(&acc_empty[ab]), 0));
@@ -381,7 +393,7 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
         float tl[4] = {0.f, 0.f, 0.f, 0.f};                      // TOK: this pixel's four token logits
 #pragma unroll
         for (int c = 0; c < 32; ++c) {
-          float x = fmaf(__uint_as_float(u[c]), 1.0f / 2048.0f, __uint_as_float(v[c]));
+          float x = P1 ? __uint_as_float(v[c]) : fmaf(__uint_as_float(u[c]), 1.0f / 2048.0f, __uint_as_float(v[c]));
           if (EPI == EPI_TOK) {                                  // squeeze: no bias, ReLU; logits from the ReLU-ed value
             x = fmaxf(x, 0.f);
             const float4 wt = *reinterpret_cast<const float4*>(wtok_s + c * 4);
@@ -403,7 +415,8 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
           o1.x += bia1.x; o1.y += bia1.y; o1.z += bia1.z; o1.w += bia1.w;
           if (e.res) {
             float4 x0, x1;
-            if (e.res_split) join8(ra[g], rb[g], x0, x1); else { x0 = as_f4(ra[g]); x1 = as_f4(rb[g]); }
+            if (e.res_split) { if (P1) half8(ra[g], x0, x1); else join8(ra[g], rb[g], x0, x1); }
+            else { x0 = as_f4(ra[g]); x1 = as_f4(rb[g]); }
             o0.x += x0.x; o0.y += x0.y; o0.z += x0.z; o0.w += x0.w;
             o1.x += x1.x; o1.y += x1.y; o1.z += x1.z; o1.w += x1.w;
           }
@@ -412,7 +425,12 @@ conv_tc3_kernel(const __grid_constant__ CUtensorMap tmA0h, const __grid_constant
             o1.x = fmaxf(o1.x, 0.f); o1.y = fmaxf(o1.y, 0.f); o1.z = fmaxf(o1.z, 0.f); o1.w = fmaxf(o1.w, 0.f);
           }
           if (ok[g]) {
-            if (EPI == EPI_SPLIT || (EPI == EPI_TOK && e.out_split)) {
+            if (P1 && e.out_split) {                             // one FP16 plane (pixel-shuffle as below)
+              uint16_t* o16 = reinterpret_cast<uint16_t*>(e.out);
+              const size_t off = rowoff[g] + (e.ps ? ((size_t)(j >> 1) * (2 * e.OW) + (j & 1)) * 32 : (size_t)j * 32);
+              *reinterpret_cast<uint4*>(o16 + off) = make_uint4(pack_f16x2_sat(o0.x, o0.y), pack_f16x2_sat(o0.z, o0.w),
+                                                                pack_f16x2_sat(o1.x, o1.y), pack_f16x2_sat(o1.z, o1.w));
+            } else if (!P1 && (EPI == EPI_SPLIT || (EPI == EPI_TOK && e.out_split))) {
               uint4 h, l;
               split8(o0, o1, h, l);
               uint16_t* o16 = reinterpret_cast<uint16_t*>(e.out);
@@ -545,9 +563,10 @@ int act_map(CUtensorMap* out, const void* ptr, int C, int W, int H, int N, int b
   *out = m;
   return 0;
 }
-// filter planes h_w / l_w: [2][Cout][K] FP16 with `plane_bytes` between the planes, read in {32 k, NT rows, 2 planes} boxes
-int filt_map(CUtensorMap* out, const void* ptr, int K, int Cout, long long plane_bytes, int NT) {
-  Key3 key{ptr, {K, Cout, plane_bytes, NT, -3}};
+// filter planes h_w / l_w: [2][Cout][K] FP16 with `plane_bytes` between the planes, read in {32 k, NT rows, `planes`} boxes
+// (planes = 2: [h_w ; l_w], 1: h_w alone)
+int filt_map(CUtensorMap* out, const void* ptr, int K, int Cout, long long plane_bytes, int NT, int planes) {
+  Key3 key{ptr, {K, Cout, plane_bytes, NT, -1 - planes}};
   {
     std::lock_guard<std::mutex> lk(g_mu3);
     auto it = g_maps3.find(key);
@@ -555,9 +574,9 @@ int filt_map(CUtensorMap* out, const void* ptr, int K, int Cout, long long plane
   }
   EncodeTiledFn3 enc = get_encode3();
   if (!enc) return DH_E_VARIANT;
-  cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)Cout, 2};
+  cuuint64_t dims[3] = {(cuuint64_t)K, (cuuint64_t)Cout, (cuuint64_t)planes};
   cuuint64_t strides[2] = {(cuuint64_t)K * 2, (cuuint64_t)plane_bytes};
-  cuuint32_t box[3] = {32, (cuuint32_t)NT, 2};
+  cuuint32_t box[3] = {32, (cuuint32_t)NT, (cuuint32_t)planes};
   cuuint32_t estr[3] = {1, 1, 1};
   CUtensorMap m;
   const CUresult r = enc(&m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(ptr), dims, strides, box, estr,
@@ -574,10 +593,10 @@ int filt_map(CUtensorMap* out, const void* ptr, int K, int Cout, long long plane
 
 constexpr uint32_t T3_SMEM_MAX = 232448 - 1024;         // 227 KB opt-in limit minus the static shared memory (barriers)
 
-template <int NT, int KS, int SD, int EPI, bool RES, int CG>
+template <int NT, int KS, int SD, int EPI, bool RES, int CG, bool P1>
 int launch3k(const CUtensorMap* A, const CUtensorMap& Bm, const T3Args& e, uint32_t smem, dim3 grid, cudaStream_t s) {
-  using Cfg = T3Cfg<NT, RES, CG>;
-  auto kern = conv_tc3_kernel<NT, KS, SD, EPI, RES, CG>;
+  using Cfg = T3Cfg<NT, RES, CG, P1>;
+  auto kern = conv_tc3_kernel<NT, KS, SD, EPI, RES, CG, P1>;
   cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3_SMEM_MAX);
   if (err != cudaSuccess) return (int)err;
   cudaLaunchConfig_t cfg = {};
@@ -595,27 +614,40 @@ int launch3k(const CUtensorMap* A, const CUtensorMap& Bm, const T3Args& e, uint3
   DH_CHECK_LAUNCH();
   return 0;
 }
-// the instantiations the network uses: tok = 1x1 / NT 32 / single CTA; everything else by (NT, K, stride, output format)
-template <int NT, bool RES, int CG>
+// the instantiations the network uses: tok = 1x1 / NT 32 / single CTA; everything else by (NT, K, stride, output format).
+// P1: one instantiation per geometry, the output format (one FP16 plane or fp32) is read at run time (T3Args::out_split)
+template <int NT, bool RES, int CG, bool P1>
 int launch3(const CUtensorMap* A, const CUtensorMap& Bm, const T3Args& e, int ks, int stride, int epi, uint32_t smem, dim3 grid, cudaStream_t s) {
   if (epi == EPI_TOK) {
-    if constexpr (NT == 32 && CG == 1) return launch3k<32, 1, 1, EPI_TOK, RES, 1>(A, Bm, e, smem, grid, s);
+    if constexpr (NT == 32 && CG == 1) return launch3k<32, 1, 1, EPI_TOK, RES, 1, P1>(A, Bm, e, smem, grid, s);
     return DH_E_SHAPE;
   }
-  if (stride == 2) {
-    if (epi == EPI_SPLIT) return ks == 3 ? launch3k<NT, 3, 2, EPI_SPLIT, RES, CG>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 2, EPI_SPLIT, RES, CG>(A, Bm, e, smem, grid, s);
-    return ks == 3 ? launch3k<NT, 3, 2, EPI_F32, RES, CG>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 2, EPI_F32, RES, CG>(A, Bm, e, smem, grid, s);
+  if constexpr (P1) {
+    if (stride == 2) return ks == 3 ? launch3k<NT, 3, 2, EPI_SPLIT, RES, CG, true>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 2, EPI_SPLIT, RES, CG, true>(A, Bm, e, smem, grid, s);
+    return ks == 3 ? launch3k<NT, 3, 1, EPI_SPLIT, RES, CG, true>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 1, EPI_SPLIT, RES, CG, true>(A, Bm, e, smem, grid, s);
+  } else {
+    if (stride == 2) {
+      if (epi == EPI_SPLIT) return ks == 3 ? launch3k<NT, 3, 2, EPI_SPLIT, RES, CG, false>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 2, EPI_SPLIT, RES, CG, false>(A, Bm, e, smem, grid, s);
+      return ks == 3 ? launch3k<NT, 3, 2, EPI_F32, RES, CG, false>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 2, EPI_F32, RES, CG, false>(A, Bm, e, smem, grid, s);
+    }
+    if (epi == EPI_SPLIT) return ks == 3 ? launch3k<NT, 3, 1, EPI_SPLIT, RES, CG, false>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 1, EPI_SPLIT, RES, CG, false>(A, Bm, e, smem, grid, s);
+    return ks == 3 ? launch3k<NT, 3, 1, EPI_F32, RES, CG, false>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 1, EPI_F32, RES, CG, false>(A, Bm, e, smem, grid, s);
   }
-  if (epi == EPI_SPLIT) return ks == 3 ? launch3k<NT, 3, 1, EPI_SPLIT, RES, CG>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 1, EPI_SPLIT, RES, CG>(A, Bm, e, smem, grid, s);
-  return ks == 3 ? launch3k<NT, 3, 1, EPI_F32, RES, CG>(A, Bm, e, smem, grid, s) : launch3k<NT, 1, 1, EPI_F32, RES, CG>(A, Bm, e, smem, grid, s);
 }
-template <bool RES, int CG>
+template <bool RES, int CG, bool P1>
 int launch3n(int NT, const CUtensorMap* A, const CUtensorMap& Bm, const T3Args& e, int ks, int stride, int epi, uint32_t smem, dim3 grid, cudaStream_t s) {
   switch (NT) {
-    case 128: return launch3<128, RES, CG>(A, Bm, e, ks, stride, epi, smem, grid, s);
-    case 64: return launch3<64, RES, CG>(A, Bm, e, ks, stride, epi, smem, grid, s);
-    default: return launch3<32, RES, CG>(A, Bm, e, ks, stride, epi, smem, grid, s);
+    case 128: return launch3<128, RES, CG, P1>(A, Bm, e, ks, stride, epi, smem, grid, s);
+    case 64: return launch3<64, RES, CG, P1>(A, Bm, e, ks, stride, epi, smem, grid, s);
+    default: return launch3<32, RES, CG, P1>(A, Bm, e, ks, stride, epi, smem, grid, s);
   }
+}
+template <bool RES>
+int launch3c(int cg, bool p1, int NT, const CUtensorMap* A, const CUtensorMap& Bm, const T3Args& e, int ks, int stride, int epi, uint32_t smem,
+             dim3 grid, cudaStream_t s) {
+  if (p1) return launch3n<RES, 1, true>(NT, A, Bm, e, ks, stride, epi, smem, grid, s);        // no CTA pairs in the single-plane form
+  return cg == 2 ? launch3n<RES, 2, false>(NT, A, Bm, e, ks, stride, epi, smem, grid, s)
+                 : launch3n<RES, 1, false>(NT, A, Bm, e, ks, stride, epi, smem, grid, s);
 }
 }  // namespace
 
@@ -624,7 +656,7 @@ bool dh_conv_tc3_eligible(const Conv3Args& a) {
                     (a.K == 1 || a.K == 3) && a.C0 > 0 && a.C0 % 32 == 0 && a.C1 % 32 == 0 && (a.C1 == 0 || a.in1) &&
                     (a.Cout == 32 || a.Cout == 64 || a.Cout == 128 || a.Cout == 256) && a.inH >= 1 && a.inW >= 1 && a.N >= 1;
   if (!base) return false;
-  if (a.ps) return a.Cout == 128 && a.res == nullptr && !a.out_split && a.K == 3;
+  if (a.ps) return a.Cout == 128 && a.res == nullptr && (!a.out_split || a.h16) && a.K == 3;
   if (a.tok) return a.Cout == 32 && a.K == 1 && a.stride == 1 && a.wtok && a.partials && !a.res && !a.bias;
   return true;
 }
@@ -651,11 +683,14 @@ int dh_launch_conv_tc3(const Conv3Args& a, cudaStream_t s) {
   const size_t plane0 = a.in0_plane ? (size_t)a.in0_plane : (size_t)a.N * a.inH * a.inW * a.C0;
   const size_t plane1 = a.in1_plane ? (size_t)a.in1_plane : (size_t)a.N * a.inH * a.inW * a.C1;
   int rc = act_map(&A[0], a.in0, a.C0, a.inW, a.inH, a.N, hw, hh, a.stride);
-  if (!rc) rc = act_map(&A[1], reinterpret_cast<const uint16_t*>(a.in0) + plane0, a.C0, a.inW, a.inH, a.N, hw, hh, a.stride);
+  if (rc) return rc;
+  A[1] = A[0];                                                               // h16: no lo planes
+  if (!a.h16) rc = act_map(&A[1], reinterpret_cast<const uint16_t*>(a.in0) + plane0, a.C0, a.inW, a.inH, a.N, hw, hh, a.stride);
   if (rc) return rc;
   if (a.C1) {
     rc = act_map(&A[2], a.in1, a.C1, a.inW, a.inH, a.N, hw, hh, a.stride);
-    if (!rc) rc = act_map(&A[3], reinterpret_cast<const uint16_t*>(a.in1) + plane1, a.C1, a.inW, a.inH, a.N, hw, hh, a.stride);
+    A[3] = A[2];
+    if (!rc && !a.h16) rc = act_map(&A[3], reinterpret_cast<const uint16_t*>(a.in1) + plane1, a.C1, a.inW, a.inH, a.N, hw, hh, a.stride);
     if (rc) return rc;
   } else { A[2] = A[0]; A[3] = A[1]; }
   // CTA pairs: DAHITRA_TC3_CG = 0 (default) never — measured 15-50 % slower on every layer of this network, see DESIGN.md — | 1 on the N = 128 tiles and the K = 1152 -> 32 head conv | 2 always
@@ -663,8 +698,9 @@ int dh_launch_conv_tc3(const Conv3Args& a, cudaStream_t s) {
   static const bool env_stream = [] { const char* v = getenv("DAHITRA_TC3_STREAM"); return v && v[0] == '1'; }();   // A/B switch
   const int mtiles = dh_cdiv(a.inW / a.stride, T3_TW) * dh_cdiv(a.inH / a.stride, T3_TH) * a.N;
   int cg = a.tok ? 1 : (a.cg ? a.cg : (env_cg == 2 ? 2 : (env_cg == 1 && (NT == 128 || (a.Cout == 32 && K >= 1152)) ? 2 : 1)));
+  DH_REQUIRE(!(a.h16 && cg == 2), DH_E_VARIANT);                           // the single-plane form has no CTA-pair variant
   if (mtiles < 2) cg = 1;
-  rc = filt_map(&Bm, a.wt16, K, a.Cout, a.wt_plane_bytes, NT / cg);
+  rc = filt_map(&Bm, a.wt16, K, a.Cout, a.wt_plane_bytes, NT / cg, a.h16 ? 1 : 2);
   if (rc) return rc;
   T3Args e;
   e.bias = a.bias; e.res = a.res; e.out = a.out; e.wtok = a.wtok; e.partials = a.partials;
@@ -678,28 +714,28 @@ int dh_launch_conv_tc3(const Conv3Args& a, cudaStream_t s) {
   e.res_plane = a.res_plane ? a.res_plane : (long long)a.N * e.OH * e.OW * a.Cout;
   e.out_plane = a.out_plane ? a.out_plane : (long long)a.N * e.OH * e.OW * a.Cout;
   e.halo_plane_bytes = (uint32_t)(hw * hh * 64);
-  const int epi = a.tok ? EPI_TOK : (a.out_split ? EPI_SPLIT : EPI_F32);
+  const int epi = a.tok ? EPI_TOK : ((a.out_split || a.h16) ? EPI_SPLIT : EPI_F32);
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int slots = sms / cg;                                                // persistent: one CTA (pair) per SM (TPC)
   const int nwork = e.ntiles < slots ? e.ntiles : slots;
   dim3 grid((unsigned)(nwork * cg), 1, 1);
-  // resident filter when the whole [h_w ; l_w] image (a CTA of a pair: its half) fits next to two halo buffers, and every
-  // CTA walks enough tiles to amortise loading it (otherwise the streaming ring, whose first MMA starts after one stage)
-  const uint32_t w_bytes = (uint32_t)K * (uint32_t)a.Cout * 4u / (uint32_t)cg;   // = ncout_tiles * cchunks * taps * B_TAP
+  // resident filter when the whole [h_w ; l_w] image (h16: h_w; a CTA of a pair: its half) fits next to two halo buffers, and
+  // every CTA walks enough tiles to amortise loading it (otherwise the streaming ring, whose first MMA starts after one stage)
+  const uint32_t w_bytes = (uint32_t)K * (uint32_t)a.Cout * (a.h16 ? 2u : 4u) / (uint32_t)cg;   // = ncout_tiles * cchunks * taps * B_TAP
+  const uint32_t halo = a.h16 ? T3_PLANE : T3_HALO;                        // one halo buffer
   const uint32_t fixed = 8 * 4096 + 1024 + (a.tok ? 512 + 2 * 2176 : 0);   // epilogue staging (8 warps) + alignment slack (+ tok scratch)
-  const bool res_ok = w_bytes + 2 * T3_HALO + fixed <= T3_SMEM_MAX && !a.force_stream && !env_stream && e.ntiles >= 2 * nwork;
+  const bool res_ok = w_bytes + 2 * halo + fixed <= T3_SMEM_MAX && !a.force_stream && !env_stream && e.ntiles >= 2 * nwork;
   if (res_ok) {
-    int hb = (int)((T3_SMEM_MAX - fixed - w_bytes) / T3_HALO);
+    int hb = (int)((T3_SMEM_MAX - fixed - w_bytes) / halo);
     e.hb = hb > T3_MAX_HB ? T3_MAX_HB : hb;
-    const uint32_t smem = (uint32_t)e.hb * T3_HALO + w_bytes + fixed;
-    return cg == 2 ? launch3n<true, 2>(NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s)
-                   : launch3n<true, 1>(NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s);
+    const uint32_t smem = (uint32_t)e.hb * halo + w_bytes + fixed;
+    return launch3c<true>(cg, a.h16, NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s);
   }
   e.hb = T3_MAX_HB;
-  const uint32_t ring = NT == 128 ? T3Cfg<128, false>::RING_BYTES : (NT == 64 ? T3Cfg<64, false>::RING_BYTES : T3Cfg<32, false>::RING_BYTES);
-  const uint32_t smem = T3_MAX_HB * T3_HALO + ring + fixed;               // the pair's ring has twice the stages of half the size
-  return cg == 2 ? launch3n<false, 2>(NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s)
-                 : launch3n<false, 1>(NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s);
+  const uint32_t ring = a.h16 ? (NT == 128 ? T3Cfg<128, false, 1, true>::RING_BYTES : (NT == 64 ? T3Cfg<64, false, 1, true>::RING_BYTES : T3Cfg<32, false, 1, true>::RING_BYTES))
+                              : (NT == 128 ? T3Cfg<128, false>::RING_BYTES : (NT == 64 ? T3Cfg<64, false>::RING_BYTES : T3Cfg<32, false>::RING_BYTES));
+  const uint32_t smem = T3_MAX_HB * halo + ring + fixed;                  // the pair's ring has twice the stages of half the size
+  return launch3c<false>(cg, a.h16, NT, A, Bm, e, a.K, a.stride, epi, smem, grid, s);
 }

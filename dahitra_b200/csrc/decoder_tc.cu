@@ -175,7 +175,7 @@ template <int HEADS, bool X3>
 __global__ void __launch_bounds__(PDT_ROWS * PdtCfg<X3>::G, 1)
 pixel_decoder_tc_kernel(const float* __restrict__ x, const float* __restrict__ pos, const float* __restrict__ tables,
                         const float* __restrict__ pack, int npix, int w, int depth, const float* __restrict__ skip,
-                        int skip_up, float* __restrict__ out, long long out_split_plane) {
+                        int skip_up, float* __restrict__ out, long long out_split_plane, int h16) {
   using Cfg = PdtCfg<X3>;
   constexpr int H4 = HEADS * 4;
   constexpr uint32_t IDESC_S = umma_idesc_tf32(128, H4);
@@ -251,7 +251,12 @@ pixel_decoder_tc_kernel(const float* __restrict__ x, const float* __restrict__ p
     const int r = g * 4 + r8, pr = pw0 + r;
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
     if (pr < npix) {
-      v = ldg4(x + ((size_t)img * npix + pr) * 32 + c8 * 4);
+      if (h16) {                                                        // x is one FP16 plane: 4 channels = 8 bytes
+        const uint2 u = __ldg(reinterpret_cast<const uint2*>(reinterpret_cast<const uint16_t*>(x) + ((size_t)img * npix + pr) * 32 + c8 * 4));
+        v = make_float4(f16_lo(u.x), f16_hi(u.x), f16_lo(u.y), f16_hi(u.y));
+      } else {
+        v = ldg4(x + ((size_t)img * npix + pr) * 32 + c8 * 4);
+      }
       if (pos) { const float4 q = ldg4(pos + (size_t)pr * 32 + c8 * 4); v.x += q.x; v.y += q.y; v.z += q.z; v.w += q.w; }
     }
     *reinterpret_cast<float4*>(io + r * 32 + ((c8 ^ (r & 7)) << 2)) = v;
@@ -439,9 +444,9 @@ pixel_decoder_tc_kernel(const float* __restrict__ x, const float* __restrict__ p
   for (int q = 0; q < 8; ++q)
     *reinterpret_cast<float4*>(io + lane * 32 + ((q ^ (lane & 7)) << 2)) = make_float4(xr[q * 2].x, xr[q * 2].y, xr[q * 2 + 1].x, xr[q * 2 + 1].y);
   __syncwarp();
-  if (out_split_plane) {
-    // split16 planes for conv_tc3.cu (hi = f16(o), lo = f16(2^11 (o - hi))): 4 lanes x 8 channels per pixel row, 16 bytes per
-    // lane and plane
+  if (out_split_plane || h16) {
+    // split16 planes for conv_tc3.cu (hi = f16(o), lo = f16(2^11 (o - hi))), or h16: hi alone, and the skip is one FP16 plane
+    // too: 4 lanes x 8 channels per pixel row, 16 bytes per lane and plane
     const int c4 = lane & 3, r4 = lane >> 2;
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
@@ -451,23 +456,32 @@ pixel_decoder_tc_kernel(const float* __restrict__ x, const float* __restrict__ p
         float4 o1 = *reinterpret_cast<const float4*>(io + r * 32 + (((2 * c4 + 1) ^ (r & 7)) << 2));
         if (skip) {
           const int py = pr / w, px = pr - py * w;
-          const float* sp = (skip_up == 2)
-              ? skip + (((size_t)img * (npix / w / 2) + (py >> 1)) * (w >> 1) + (px >> 1)) * 32
-              : skip + ((size_t)img * npix + pr) * 32;
-          const float4 v0 = ldg4(sp + c4 * 8), v1 = ldg4(sp + c4 * 8 + 4);
+          const size_t so = (skip_up == 2) ? (((size_t)img * (npix / w / 2) + (py >> 1)) * (w >> 1) + (px >> 1)) * 32
+                                           : ((size_t)img * npix + pr) * 32;
+          float4 v0, v1;
+          if (h16) {
+            const uint4 u = __ldg(reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(skip) + so + c4 * 8));
+            v0 = make_float4(f16_lo(u.x), f16_hi(u.x), f16_lo(u.y), f16_hi(u.y));
+            v1 = make_float4(f16_lo(u.z), f16_hi(u.z), f16_lo(u.w), f16_hi(u.w));
+          } else {
+            v0 = ldg4(skip + so + c4 * 8); v1 = ldg4(skip + so + c4 * 8 + 4);
+          }
           o0.x += v0.x; o0.y += v0.y; o0.z += v0.z; o0.w += v0.w;
           o1.x += v1.x; o1.y += v1.y; o1.z += v1.z; o1.w += v1.w;
         }
-        uint4 hi, lo;
+        uint4 hi;
         hi.x = pack_f16x2_sat(o0.x, o0.y); hi.y = pack_f16x2_sat(o0.z, o0.w); hi.z = pack_f16x2_sat(o1.x, o1.y); hi.w = pack_f16x2_sat(o1.z, o1.w);
-        lo.x = pack_f16x2_sat((o0.x - f16_lo(hi.x)) * 2048.f, (o0.y - f16_hi(hi.x)) * 2048.f);
-        lo.y = pack_f16x2_sat((o0.z - f16_lo(hi.y)) * 2048.f, (o0.w - f16_hi(hi.y)) * 2048.f);
-        lo.z = pack_f16x2_sat((o1.x - f16_lo(hi.z)) * 2048.f, (o1.y - f16_hi(hi.z)) * 2048.f);
-        lo.w = pack_f16x2_sat((o1.z - f16_lo(hi.w)) * 2048.f, (o1.w - f16_hi(hi.w)) * 2048.f);
         uint16_t* o16 = reinterpret_cast<uint16_t*>(out);
         const size_t off = ((size_t)img * npix + pr) * 32 + c4 * 8;
         *reinterpret_cast<uint4*>(o16 + off) = hi;
-        *reinterpret_cast<uint4*>(o16 + off + (size_t)out_split_plane) = lo;
+        if (out_split_plane) {
+          uint4 lo;
+          lo.x = pack_f16x2_sat((o0.x - f16_lo(hi.x)) * 2048.f, (o0.y - f16_hi(hi.x)) * 2048.f);
+          lo.y = pack_f16x2_sat((o0.z - f16_lo(hi.y)) * 2048.f, (o0.w - f16_hi(hi.y)) * 2048.f);
+          lo.z = pack_f16x2_sat((o1.x - f16_lo(hi.z)) * 2048.f, (o1.y - f16_hi(hi.z)) * 2048.f);
+          lo.w = pack_f16x2_sat((o1.z - f16_lo(hi.w)) * 2048.f, (o1.w - f16_hi(hi.w)) * 2048.f);
+          *reinterpret_cast<uint4*>(o16 + off + (size_t)out_split_plane) = lo;
+        }
       }
     }
   } else {
@@ -498,12 +512,12 @@ pixel_decoder_tc_kernel(const float* __restrict__ x, const float* __restrict__ p
 
 template <int HEADS, bool X3>
 int launch_pdt(dim3 grid, const float* x, const float* pos, const float* tables, const float* pack, int npix, int w, int depth,
-               const float* skip, int skip_up, float* out, long long osp, cudaStream_t s) {
+               const float* skip, int skip_up, float* out, long long osp, int h16, cudaStream_t s) {
   cudaError_t e = cudaFuncSetAttribute(pixel_decoder_tc_kernel<HEADS, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (int)PdtCfg<X3>::SMEM);
   if (e != cudaSuccess) return (int)e;
   return dh_launch(pixel_decoder_tc_kernel<HEADS, X3>, grid, dim3(PDT_ROWS * PdtCfg<X3>::G), (size_t)PdtCfg<X3>::SMEM, s, x, pos, tables, pack,
-                   npix, w, depth, skip, skip_up, out, (long long)osp);
+                   npix, w, depth, skip, skip_up, out, (long long)osp, h16);
 }
 }  // namespace
 
@@ -519,11 +533,14 @@ int dh_launch_decoder_tables_tc(const float* mem, int B, int first_call, int nca
   return dh_launch(decoder_tables_tc_kernel, grid, dim3(128), (size_t)smem, s, mem, B, first_call, dec, heads, tables, depth);
 }
 
-// x3: bit 0 = error-compensated 3xTF32; bit 8 (x3 | 256): `out` receives split16 planes (conv_tc3.cu's input format)
+// x3: bit 0 = error-compensated 3xTF32; bit 8 (x3 | 256): `out` receives split16 planes (conv_tc3.cu's input format);
+// bit 9 (x3 | 512): x, skip and out are one FP16 plane each (the h16 mode)
 int dh_launch_pixel_decoder_tc(const float* x, const float* pos, const float* tables, const float* pack, int nimg, int h,
                                int w, int heads, int depth, const float* skip, int skip_up, int x3, float* out,
                                cudaStream_t s) {
   const long long osp = (x3 & 256) ? (long long)nimg * h * w * 32 : 0;
+  const int h16 = (x3 & 512) ? 1 : 0;
+  DH_REQUIRE(!(h16 && osp), DH_E_VARIANT);
   x3 &= 1;
   DH_REQUIRE(x && tables && pack && out, DH_E_NULL);
   DH_REQUIRE(nimg > 0 && h > 0 && w > 0 && depth >= 1 && (heads == 4 || heads == 8), DH_E_SHAPE);
@@ -533,8 +550,8 @@ int dh_launch_pixel_decoder_tc(const float* x, const float* pos, const float* ta
   const int npix = h * w;
   dim3 grid(dh_cdiv(npix, PDT_ROWS * PdtCfg<true>::G), nimg);
   if (heads == 4)
-    return x3 ? launch_pdt<4, true>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, s)
-              : launch_pdt<4, false>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, s);
-  return x3 ? launch_pdt<8, true>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, s)
-            : launch_pdt<8, false>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, s);
+    return x3 ? launch_pdt<4, true>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, h16, s)
+              : launch_pdt<4, false>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, h16, s);
+  return x3 ? launch_pdt<8, true>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, h16, s)
+            : launch_pdt<8, false>(grid, x, pos, tables, pack, npix, w, depth, skip, skip_up, out, osp, h16, s);
 }

@@ -228,10 +228,12 @@ extern "C" int dahitra_conv2d_split(const void* in0, const void* in1, int C0, in
                                     const void* res, int res_split, int relu, void* out, int out_split, int mode,
                                     const float* w_tok, float* partials, void* stream) {
   DH_REQUIRE(wt, DH_E_NULL);
-  const int sched = mode & ~3;                                       // scheduling bits (do not change results)
+  const int h16 = (mode & 128) ? 1 : 0;                              // storage format: one FP16 plane instead of split16
+  const int sched = mode & ~(3 | 128);                               // scheduling bits (do not change results)
   mode &= 3;
   DH_REQUIRE(mode <= 2 && !(sched & ~(16 | 32 | 64)), DH_E_VARIANT);
   Conv3Args a{};
+  a.h16 = h16;
   a.cg = (sched & 32) ? 2 : ((sched & 16) ? 1 : 0);
   a.force_stream = (sched & 64) ? 1 : 0;
   a.in0 = in0; a.in1 = in1; a.C0 = C0; a.C1 = C1; a.N = N; a.inH = inH; a.inW = inW; a.in0_plane = in0_plane; a.in1_plane = in1_plane;
@@ -245,6 +247,13 @@ extern "C" int dahitra_conv2d_split(const void* in0, const void* in1, int C0, in
 extern "C" int dahitra_classifier(const float* in, int N, int H, int W, int nc, const float* w, const float* bias,
                                   float* logits, unsigned char* argmax_u8, void* stream) {
   return dh_launch_classifier(in, N, H, W, nc, w, bias, logits, argmax_u8, (cudaStream_t)stream);
+}
+extern "C" int dahitra_maxpool3x3s2_h16(const void* in, int N, int H, int W, int C, void* out, void* stream) {
+  return dh_launch_maxpool_h16(in, N, H, W, C, out, (cudaStream_t)stream);
+}
+extern "C" int dahitra_classifier_h16(const void* in, int N, int H, int W, int nc, const float* w, const float* bias,
+                                      float* logits, unsigned char* argmax_u8, void* stream) {
+  return dh_launch_classifier_h16(in, N, H, W, nc, w, bias, logits, argmax_u8, (cudaStream_t)stream);
 }
 
 // ----------------------------------------------------------------------------------------------------
@@ -336,6 +345,10 @@ AuxStreams* aux_streams() {
 //   split16: F2, P2, T4*, F4, T8*, F8, P8, T16*, F16, Y20, O2, decoder outputs read by a conv (XD; OUT of levels 4, 3),
 //            XS in the xBD variant (read by conv_decode)
 //   fp32:    XS (LEVIR: read by the decoder), DX, OUT of level 5 (a decoder skip), C4, C3, C2, logits
+// The same sequence runs the h16 mode (DH_FLAG_ACT_H16): EVERY tensor listed above is stored as one FP16 plane (hi alone, 2 bytes
+// per element, in half the buffer), the convolutions take the single-plane form of conv_tc3 (one MMA per (tap, chunk, K step)),
+// the max pools and the classifier read FP16; the tokenizer partials, token memories and decoder tables stay fp32.  The
+// algorithmic byte counts of the profiler use 2 bytes per element for those tensors (and for the h_w filter plane).
 // ----------------------------------------------------------------------------------------------------
 namespace {
 int forward_split(const Plan& p, const void* const* weights, const float* x1, const float* x2, long long x_batch_stride,
@@ -345,6 +358,8 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
   auto Wt = [&](int slot) { return (const float*)weights[slot]; };
   const int N2 = 2 * B;
   const int h2 = H / 2, w2 = W / 2, h4 = H / 4, w4 = W / 4, h8 = H / 8, w8 = W / 8, h16 = H / 16, w16 = W / 16;
+  const bool one = (flags & DH_FLAG_ACT_H16) != 0;     // one FP16 plane per tensor (every res / out below is then FP16)
+  const double eb = one ? 2.0 : 4.0;                   // stored bytes per element of the tensors listed above
   // conv over split16 inputs.  wts: the filter's *_WT (or _PSWT) slot; in_plane: elements between the hi / lo planes of in0 / in1
   auto conv3 = [&](const char* name, const float* in0, const float* in1, int C0, int C1, long long in_plane, int N, int inH, int inW,
                    int K, int stride, int Cout, int wts, int bslot, const float* res, int res_split, int relu, float* out,
@@ -354,14 +369,15 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
     a.K = K; a.stride = stride; a.Cout = Cout;
     const size_t plane = (size_t)Cout * K * K * (C0 + C1);
     a.wt16 = Wt(wts) + 3 * plane; a.wt_plane_bytes = (long long)plane * 4;
-    a.bias = bslot >= 0 ? Wt(bslot) : nullptr; a.res = res; a.res_split = res_split; a.relu = relu; a.out = out; a.out_split = out_split;
-    a.ps = ps;
+    a.bias = bslot >= 0 ? Wt(bslot) : nullptr; a.res = res; a.res_split = one ? 1 : res_split; a.relu = relu; a.out = out;
+    a.out_split = one ? 1 : out_split;
+    a.ps = ps; a.h16 = one;
     const int rc = dh_launch_conv_tc3(a, s);
     if (rc != 0) return rc;
     const double OH = (double)inH / stride, OW = (double)inW / stride, Cin = C0 + C1;
     const double cout_alg = ps ? 32.0 : Cout, up = ps ? 2.0 : 1.0;       // as written: a 3x3 conv 32 -> 32 on the upsampled map
     const double fl = 2.0 * N * OH * up * OW * up * cout_alg * K * K * Cin;
-    const double by = 4.0 * ((double)N * inH * inW * Cin + (double)N * OH * up * OW * up * cout_alg * (res ? 2 : 1) + (double)K * K * Cin * cout_alg);
+    const double by = eb * ((double)N * inH * inW * Cin + (double)N * OH * up * OW * up * cout_alg * (res ? 2 : 1) + (double)K * K * Cin * cout_alg);
     prof_mark(s, name, fl, by);
     return 0;
   };
@@ -378,13 +394,17 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
   const size_t f2_half = (size_t)B * h2 * w2 * 64;
   const long long f2_plane = (long long)N2 * h2 * w2 * 64;
   float* F2post = reinterpret_cast<float*>(H16(F2) + f2_half);             // hi plane of the post images
-  const double stem_fl = 2.0 * B * h2 * w2 * 64 * 147, stem_by = 4.0 * B * ((double)3 * H * W + (double)h2 * w2 * 64);
-  const int stem_mode = ((flags & DH_FLAG_TC_3XTF32) ? 2 : 3) | 256;
+  const double stem_fl = 2.0 * B * h2 * w2 * 64 * 147;
+  const double stem_by = one ? B * (4.0 * 3 * H * W + 2.0 * h2 * w2 * 64) : 4.0 * B * ((double)3 * H * W + (double)h2 * w2 * 64);
+  const int stem_mode = one ? 3 | 512 : ((flags & DH_FLAG_TC_3XTF32) ? 2 : 3) | 256;
   // one launch over both image sets (pre images first): x2 is addressed through a second tensor map
   DH_STEP("stem", 2.0 * stem_fl, 2.0 * stem_by,
           dh_launch_stem_tc(x1, x_batch_stride, B, H, W, Wt(DH_W_STEM_WTC), Wt(DH_W_STEM_B), F2, stem_mode, s, f2_plane, x2));
   float* P2 = ws + p.p2;
-  DH_STEP("maxpool_2", 0.0, 4.0 * N2 * 64 * ((double)h2 * w2 + (double)h4 * w4), dh_launch_maxpool_split(F2, N2, h2, w2, 64, P2, s));
+  auto maxpool = [&](const float* in, int hh, int ww, int C, float* out) {
+    return one ? dh_launch_maxpool_h16(in, N2, hh, ww, C, out, s) : dh_launch_maxpool_split(in, N2, hh, ww, C, out, s);
+  };
+  DH_STEP("maxpool_2", 0.0, eb * N2 * 64 * ((double)h2 * w2 + (double)h4 * w4), maxpool(F2, h2, w2, 64, P2));
   float *T4a = ws + p.t4a, *T4b = ws + p.t4b, *F4 = ws + p.f4;
   DH_CONV3("layer1.0.conv1", P2, nullptr, 64, 0, 0, N2, h4, w4, 3, 1, 64, DH_W_L1_0_C1_WT, DH_W_L1_0_C1_B, nullptr, 0, 1, T4a, 1, 0);
   DH_CONV3("layer1.0.conv2", T4a, nullptr, 64, 0, 0, N2, h4, w4, 3, 1, 64, DH_W_L1_0_C2_WT, DH_W_L1_0_C2_B, P2, 1, 1, T4b, 1, 0);
@@ -397,7 +417,7 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
   DH_CONV3("layer2.1.conv1", T8c, nullptr, 128, 0, 0, N2, h8, w8, 3, 1, 128, DH_W_L2_1_C1_WT, DH_W_L2_1_C1_B, nullptr, 0, 1, T8a, 1, 0);
   DH_CONV3("layer2.1.conv2", T8a, nullptr, 128, 0, 0, N2, h8, w8, 3, 1, 128, DH_W_L2_1_C2_WT, DH_W_L2_1_C2_B, T8c, 1, 1, F8, 1, 0);
   float* P8 = ws + p.p8;
-  DH_STEP("maxpool_8", 0.0, 4.0 * N2 * 128 * ((double)h8 * w8 + (double)h16 * w16), dh_launch_maxpool_split(F8, N2, h8, w8, 128, P8, s));
+  DH_STEP("maxpool_8", 0.0, eb * N2 * 128 * ((double)h8 * w8 + (double)h16 * w16), maxpool(F8, h8, w8, 128, P8));
   float *T16a = ws + p.t16a, *T16b = ws + p.t16b, *T16c = ws + p.t16c, *F16 = ws + p.f16;
   DH_CONV3("layer3.0.conv1", P8, nullptr, 128, 0, 0, N2, h16, w16, 3, 1, 256, DH_W_L3_0_C1_WT, DH_W_L3_0_C1_B, nullptr, 0, 1, T16a, 1, 0);
   DH_CONV3("layer3.0.down", P8, nullptr, 128, 0, 0, N2, h16, w16, 1, 1, 256, DH_W_L3_0_DS_WT, DH_W_L3_0_DS_B, nullptr, 0, 0, T16b, 1, 0);
@@ -414,6 +434,8 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
       {"squeeze_tok_3", "token_enc_3", "dec_tables_3", "decoder_3_x12", "conv_decode_3", "decoder_3_diff", "conv_layer4"}};
   float* C4 = ws + p.c4;
   const int x3 = (flags & DH_FLAG_DEC_TC_X3) ? 1 : 0;
+  // per pixel: x, pos (fp32 weights), out — h16: x and out FP16
+  auto dec_bytes_px = [&](const float* pos) { return one ? 32.0 * (2 + 2 + (pos ? 4 : 0)) : 4.0 * 32 * (pos ? 3 : 2); };
   auto level_pre = [&](int i) -> int {
     const Level& L = p.lv[i];
     const int npix = L.h * L.w;
@@ -421,15 +443,16 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
     float *XS = ws + L.xs, *XD = ws + L.xd, *DX = ws + L.dx, *PART = ws + L.part, *MEM = ws + L.mem, *TAB = ws + L.tab;
     const double inner = 64.0 * L.heads;
     const double dec_fl_px = L.depth * 2.0 * (32 * inner + 4 * inner + 4 * inner + inner * 32 + 2 * 32 * 32);
-    const double dec_by_px = 4.0 * 32 * (pos ? 3 : 2);
+    const double dec_by_px = dec_bytes_px(pos);
     const bool levir = variant == DH_VARIANT_LEVIR;
     {   // squeeze 1x1 + ReLU + tokenizer partials on the tensor cores; xs fp32 for the decoder (LEVIR) / split16 for conv_decode (xBD)
+        // (h16: FP16 for both)
       Conv3Args a{};
       a.in0 = feats[i]; a.C0 = L.cin; a.N = N2; a.inH = L.h; a.inW = L.w; a.K = 1; a.stride = 1; a.Cout = 32;
       const size_t plane = (size_t)32 * L.cin;
       a.wt16 = Wt(DH_W_LV5_SQ_WT + i) + 3 * plane; a.wt_plane_bytes = (long long)plane * 4;
-      a.out = XS; a.out_split = levir ? 0 : 1; a.tok = 1; a.wtok = wtok; a.partials = PART;
-      DH_STEP(nm[i][0], 2.0 * N2 * npix * 32 * (L.cin + 4 + 4), 4.0 * N2 * npix * (L.cin + 32.0), dh_launch_conv_tc3(a, s));
+      a.out = XS; a.out_split = (levir && !one) ? 0 : 1; a.tok = 1; a.wtok = wtok; a.partials = PART; a.h16 = one;
+      DH_STEP(nm[i][0], 2.0 * N2 * npix * 32 * (L.cin + 4 + 4), eb * N2 * npix * (L.cin + 32.0), dh_launch_conv_tc3(a, s));
     }
     const int add_tok_pos = levir ? 1 : (i == 0 ? 1 : 0);
     DH_STEP(nm[i][1], 0.0, 4.0 * N2 * L.nchunk3 * 136.0, dh_launch_token_encoder(PART, B, L.nchunk3, enc, L.heads, add_tok_pos, MEM, s));
@@ -439,7 +462,7 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
     if (levir) {
       DH_STEP(nm[i][2], 0.0, 4.0 * 3 * B * L.depth * (double)DH_TABTC_FLOATS, dh_launch_decoder_tables_tc(MEM, B, 0, 3, dec, L.heads, L.depth, TAB, s));
       DH_STEP(nm[i][3], dec_fl_px * N2 * npix, dec_by_px * N2 * npix,
-              dh_launch_pixel_decoder_tc(XS, pos, TAB, dectc, N2, L.h, L.w, L.heads, L.depth, nullptr, 1, x3 | 256, XD, s));
+              dh_launch_pixel_decoder_tc(XS, pos, TAB, dectc, N2, L.h, L.w, L.heads, L.depth, nullptr, 1, x3 | (one ? 512 : 256), XD, s));
       DH_CONV3(nm[i][4], XD, reinterpret_cast<float*>(H16(XD) + half), 32, 32, plane2, B, L.h, L.w, 3, 1, 32, DH_W_LV5_DECODE_WT + i, -1,
                nullptr, 0, 0, DX, 0, 0);
     } else {
@@ -454,15 +477,15 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
     const int npix = L.h * L.w;
     const float* pos = Wt(base[i] + 4);
     float *DX = ws + L.dx, *OUT = ws + L.out, *TAB = ws + L.tab;
-    const float* skip = (i == 0) ? nullptr : (i == 1 ? ws + p.lv[0].out : C4);     // both fp32
+    const float* skip = (i == 0) ? nullptr : (i == 1 ? ws + p.lv[0].out : C4);     // both fp32 (h16: FP16)
     const int skip_up = (i == 1) ? 2 : 1;
     const double inner = 64.0 * L.heads;
     const double dec_fl_px = L.depth * 2.0 * (32 * inner + 4 * inner + 4 * inner + inner * 32 + 2 * 32 * 32);
-    const double dec_by_px = 4.0 * 32 * (pos ? 3 : 2);
+    const double dec_by_px = dec_bytes_px(pos);
     const float* dectc = Wt(DH_W_LV5_DECTC + i);
     const float* tab2 = (variant == DH_VARIANT_LEVIR) ? TAB + (size_t)2 * B * L.depth * DH_TABTC_FLOATS : TAB;
-    const int out_split = i == 0 ? 0 : 256;                 // level 5's result is only a decoder skip; levels 4 / 3 feed conv_layer4 / 3
-    DH_STEP(nm[i][5], dec_fl_px * B * npix, (dec_by_px + (skip ? 128.0 / (skip_up * skip_up) : 0.0)) * B * npix,
+    const int out_split = one ? 512 : (i == 0 ? 0 : 256);   // level 5's result is only a decoder skip; levels 4 / 3 feed conv_layer4 / 3
+    DH_STEP(nm[i][5], dec_fl_px * B * npix, (dec_by_px + (skip ? 32.0 * eb / (skip_up * skip_up) : 0.0)) * B * npix,
             dh_launch_pixel_decoder_tc(DX, pos, tab2, dectc, B, L.h, L.w, L.heads, L.depth, skip, skip_up, x3 | out_split, OUT, s));
     if (i == 1)   // conv_layer4(up2(out_4)) -> C4 at H/4 (:1335-1336), pixel-shuffle form
       DH_CONV3(nm[i][6], OUT, nullptr, 32, 0, 0, B, L.h, L.w, 3, 1, 128, DH_W_CL4_PSWT, DH_W_CL4_PSB, nullptr, 0, 1, C4, 0, 1);
@@ -494,8 +517,10 @@ int forward_split(const Plan& p, const void* const* weights, const float* x1, co
   DH_CONV3("conv_layer2_0.0", F2, F2post, 64, 64, f2_plane, B, h2, w2, 3, 1, 128, DH_W_CL20A_WT, DH_W_CL20A_B, nullptr, 0, 1, Y20, 1, 0);
   DH_CONV3("conv_layer2_0.3", Y20, nullptr, 128, 0, 0, B, h2, w2, 3, 1, 32, DH_W_CL20B_WT, DH_W_CL20B_B, C3, 0, 0, O2, 1, 0);
   DH_CONV3("conv_layer2", O2, nullptr, 32, 0, 0, B, h2, w2, 3, 1, 128, DH_W_CL2_PSWT, DH_W_CL2_PSB, nullptr, 0, 1, C2, 0, 1);
-  DH_STEP("classifier", 2.0 * B * H * W * 9 * 32 * output_nc, 4.0 * B * H * W * (32.0 + output_nc) + (argmax_u8 ? (double)B * H * W : 0.0),
-          dh_launch_classifier(C2, B, H, W, output_nc, Wt(DH_W_CLS_W), Wt(DH_W_CLS_B), logits, argmax_u8, s));
+  DH_STEP("classifier", 2.0 * B * H * W * 9 * 32 * output_nc,
+          (one ? B * H * W * (2.0 * 32 + 4.0 * output_nc) : 4.0 * B * H * W * (32.0 + output_nc)) + (argmax_u8 ? (double)B * H * W : 0.0),
+          one ? dh_launch_classifier_h16(C2, B, H, W, output_nc, Wt(DH_W_CLS_W), Wt(DH_W_CLS_B), logits, argmax_u8, s)
+              : dh_launch_classifier(C2, B, H, W, output_nc, Wt(DH_W_CLS_W), Wt(DH_W_CLS_B), logits, argmax_u8, s));
   return 0;
 }
 }  // namespace
@@ -509,6 +534,11 @@ extern "C" int dahitra_forward(const void* const* weights, int n_weights, const 
   DH_REQUIRE(n_weights == DH_W_COUNT, DH_E_WEIGHTS);
   Plan p;
   DH_REQUIRE(variant == DH_VARIANT_LEVIR || variant == DH_VARIANT_XBD, DH_E_VARIANT);
+  if (flags & DH_FLAG_ACT_H16) {                // one-FP16-plane storage: the single-pass FP16 convs, the tcgen05 stem and decoder
+    constexpr int need = DH_FLAG_CONV_TC | DH_FLAG_TC_MAIN_F16 | DH_FLAG_TC_STRIDE2 | DH_FLAG_STEM_TC | DH_FLAG_DEC_TC;
+    DH_REQUIRE((flags & need) == need &&
+               !(flags & (DH_FLAG_ACT_SPLIT | DH_FLAG_TC_3XTF32 | DH_FLAG_TC_BF16 | DH_FLAG_CONV_TC_V1)), DH_E_VARIANT);
+  }
   DH_REQUIRE(make_plan(p, variant, B, H, W, output_nc, flags), DH_E_SHAPE);
   DH_REQUIRE(workspace_bytes >= p.total_floats * sizeof(float), DH_E_WORKSPACE);
   DH_REQUIRE(dh_aligned16(workspace), DH_E_ALIGN);
@@ -526,6 +556,8 @@ extern "C" int dahitra_forward(const void* const* weights, int n_weights, const 
     DH_REQUIRE((flags & need) == need && !(flags & (DH_FLAG_TC_BF16 | DH_FLAG_CONV_TC_V1)), DH_E_VARIANT);
     return forward_split(p, weights, x1, x2, x_batch_stride, logits, argmax_u8, ws, variant, B, H, W, output_nc, flags, s_main);
   }
+  if (flags & DH_FLAG_ACT_H16)
+    return forward_split(p, weights, x1, x2, x_batch_stride, logits, argmax_u8, ws, variant, B, H, W, output_nc, flags, s_main);
   auto Wt = [&](int slot) { return (const float*)weights[slot]; };
   const int N2 = 2 * B;
   const int h2 = H / 2, w2 = W / 2, h4 = H / 4, w4 = W / 4, h8 = H / 8, w8 = W / 8, h16 = H / 16, w16 = W / 16;

@@ -3,7 +3,8 @@
 //   * fp32 <-> split16 conversion (block tests, and the boundary of code that keeps fp32 tensors),
 //   * MaxPool2d(3, 2, 1) on a split16 NHWC tensor (reference models/networks.py:1123,1128 — the same module applied after the
 //     stem and after layer2): the order of the values is the lexicographic order of their (hi, lo) pairs, so the pool runs
-//     on packed halves and copies the winner's planes.
+//     on packed halves and copies the winner's planes;
+//   * the same pool on ONE FP16 plane (the h16 mode): a max of 16-bit values, exact.
 #include "tc_common.cuh"
 #include <cuda_fp16.h>
 
@@ -89,6 +90,40 @@ maxpool_split_kernel(const uint16_t* __restrict__ in, int N, int H, int W, int C
   *reinterpret_cast<uint4*>(out + plane_out + o) = ml;
 }
 
+// one thread = 8 channels of one output pixel (16-byte loads / stores)
+__global__ void __launch_bounds__(256)
+maxpool_h16_kernel(const uint16_t* __restrict__ in, int N, int H, int W, int C, uint16_t* __restrict__ out) {
+  const int OH = H / 2, OW = W / 2, C8 = C / 8;
+  const size_t total = (size_t)N * OH * OW * C8;
+  pdl_wait();
+  pdl_launch_dependents();
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int c8 = (int)(i % C8);
+  size_t p = i / C8;
+  const int ox = (int)(p % OW); p /= OW;
+  const int oy = (int)(p % OH);
+  const int n = (int)(p / OH);
+  __half2 m[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) m[k] = __half2half2(__ushort_as_half((unsigned short)0xFC00u));    // -inf
+#pragma unroll
+  for (int dy = -1; dy <= 1; ++dy) {
+    const int iy = 2 * oy + dy;
+    if (iy < 0 || iy >= H) continue;
+#pragma unroll
+    for (int dx = -1; dx <= 1; ++dx) {
+      const int ix = 2 * ox + dx;
+      if (ix < 0 || ix >= W) continue;
+      const uint4 v = __ldg(reinterpret_cast<const uint4*>(in + (((size_t)n * H + iy) * W + ix) * C + c8 * 8));
+      const __half2* h = reinterpret_cast<const __half2*>(&v);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) m[k] = __hmax2(m[k], h[k]);
+    }
+  }
+  *reinterpret_cast<uint4*>(out + (((size_t)n * OH + oy) * OW + ox) * C + c8 * 8) = *reinterpret_cast<const uint4*>(m);
+}
+
 int grid_for(size_t items) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
@@ -128,4 +163,12 @@ int dh_launch_maxpool_split(const void* in, int N, int H, int W, int C, void* ou
   if (e != cudaSuccess) return (int)e;
   DH_CHECK_LAUNCH();
   return 0;
+}
+int dh_launch_maxpool_h16(const void* in, int N, int H, int W, int C, void* out, cudaStream_t s) {
+  DH_REQUIRE(in && out, DH_E_NULL);
+  DH_REQUIRE(N > 0 && H >= 2 && W >= 2 && H % 2 == 0 && W % 2 == 0 && C % 8 == 0, DH_E_SHAPE);
+  DH_REQUIRE(dh_aligned16(in) && dh_aligned16(out), DH_E_ALIGN);
+  const size_t items = (size_t)N * (H / 2) * (W / 2) * (C / 8);
+  return dh_launch(maxpool_h16_kernel, dim3((unsigned)((items + 255) / 256)), dim3(256), 0, s,
+                   reinterpret_cast<const uint16_t*>(in), N, H, W, C, reinterpret_cast<uint16_t*>(out));
 }

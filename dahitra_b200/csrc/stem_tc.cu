@@ -96,7 +96,11 @@ __device__ __forceinline__ void sk_store_slice(const float (&v)[32], float* stag
       const float4 r0 = make_float4(fmaxf(o0.x + b0.x, 0.f), fmaxf(o0.y + b0.y, 0.f), fmaxf(o0.z + b0.z, 0.f), fmaxf(o0.w + b0.w, 0.f));
       const float4 r1 = make_float4(fmaxf(o1.x + b1.x, 0.f), fmaxf(o1.y + b1.y, 0.f), fmaxf(o1.z + b1.z, 0.f), fmaxf(o1.w + b1.w, 0.f));
       const size_t off = ((size_t)(t.n * OH + oy) * OW + ox) * 64 + j * 32 + c4 * 8;
-      if (split_plane) {                 // split16 planes for conv_tc3.cu: hi = f16(r), lo = f16(2^11 (r - hi))
+      if (split_plane < 0) {             // one FP16 plane (h16 mode)
+        uint4 hi;
+        hi.x = pack_f16x2_sat(r0.x, r0.y); hi.y = pack_f16x2_sat(r0.z, r0.w); hi.z = pack_f16x2_sat(r1.x, r1.y); hi.w = pack_f16x2_sat(r1.z, r1.w);
+        *reinterpret_cast<uint4*>(reinterpret_cast<uint16_t*>(out) + off) = hi;
+      } else if (split_plane) {          // split16 planes for conv_tc3.cu: hi = f16(r), lo = f16(2^11 (r - hi))
         uint4 hi, lo;
         hi.x = pack_f16x2_sat(r0.x, r0.y); hi.y = pack_f16x2_sat(r0.z, r0.w); hi.z = pack_f16x2_sat(r1.x, r1.y); hi.w = pack_f16x2_sat(r1.z, r1.w);
         lo.x = pack_f16x2_sat((r0.x - f16_lo(hi.x)) * 2048.f, (r0.y - f16_hi(hi.x)) * 2048.f);
@@ -435,15 +439,17 @@ stem_f16_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
 }  // namespace
 
 // x3: 0 = 1xTF32, 1 = 3xTF32, 2 = folded FP16, 3 = single-pass FP16; bit 8 (x3 | 256, modes 2 / 3 only): `out` receives the
-// split16 planes conv_tc3.cu consumes instead of fp32
+// split16 planes conv_tc3.cu consumes instead of fp32; bit 9 (x3 | 512, mode 3 only): one FP16 plane (the h16 mode)
 int dh_launch_stem_tc(const float* x, long long xbs, int N, int H, int W, const float* wtc, const float* b, float* out,
                       int x3, cudaStream_t s, long long split_plane_pitch, const float* x_second) {
   // x_second != NULL (forms 2 / 3): ONE launch over 2N images — N from x, then N from x_second (same strides) — writing one
   // [2N]-image output tensor: the pre and post image sets of a forward without a second launch
-  const bool split = (x3 & 256) != 0;
+  const bool split = (x3 & 256) != 0, h16 = (x3 & 512) != 0;
+  DH_REQUIRE(!(x3 & ~(255 | 256 | 512)) && !(split && h16), DH_E_VARIANT);
   x3 &= 255;
   DH_REQUIRE(!x_second || x3 == 2 || x3 == 3, DH_E_VARIANT);
   DH_REQUIRE(!split || x3 == 2 || x3 == 3, DH_E_VARIANT);
+  DH_REQUIRE(!h16 || x3 == 3, DH_E_VARIANT);
   DH_REQUIRE(x && wtc && b && out, DH_E_NULL);
   DH_REQUIRE(N > 0 && H >= 8 && W >= 8 && H % 2 == 0 && W % 2 == 0, DH_E_SHAPE);
   DH_REQUIRE(dh_aligned16(wtc) && dh_aligned16(b) && dh_aligned16(out), DH_E_ALIGN);
@@ -453,7 +459,8 @@ int dh_launch_stem_tc(const float* x, long long xbs, int N, int H, int W, const 
   const int nimg = x_second ? 2 * N : N;
   const int ntiles = tx * ty * nimg;
   // elements between the hi and lo planes: this call's own images, or the pitch of a larger tensor it writes a part of
-  const long long split_plane = split ? (split_plane_pitch ? split_plane_pitch : (long long)nimg * OH * OW * 64) : 0;
+  // (< 0: one FP16 plane)
+  const long long split_plane = h16 ? -1 : split ? (split_plane_pitch ? split_plane_pitch : (long long)nimg * OH * OW * 64) : 0;
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);

@@ -10,6 +10,8 @@ int dh_encode_tiled_f32(CUtensorMap* out, const void* ptr, int rank, const unsig
                         const unsigned long long* strides, const unsigned* box, bool swizzle128);
 int dh_encode_tiled_f32_sw(CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,
                            const unsigned long long* strides, const unsigned* box, int swizzle_bytes);
+int dh_encode_tiled_f16_sw(CUtensorMap* out, const void* ptr, int rank, const unsigned long long* dims,     // FP16 elements
+                           const unsigned long long* strides, const unsigned* box, int swizzle_bytes);
 
 namespace dhtc {
 

@@ -25,6 +25,7 @@ DH_VARIANT_LEVIR, DH_VARIANT_XBD = 0, 1
 DH_FLAG_CONV_TC, DH_FLAG_TC_3XTF32, DH_FLAG_TC_STRIDE2, DH_FLAG_DEC_TC, DH_FLAG_STEM_TC, DH_FLAG_DEC_TC_X3 = 1, 2, 4, 8, 16, 32
 DH_FLAG_CONV_TC_V1, DH_FLAG_CONV_TC_2CTA, DH_FLAG_SERIAL, DH_FLAG_TC_X3_BF16, DH_FLAG_TC_BF16 = 64, 128, 256, 512, 1024
 DH_FLAG_TC_MAIN_F16, DH_FLAG_TC_FOLD, DH_FLAG_EARLY_HEAD, DH_FLAG_ACT_SPLIT, DH_FLAG_PDL = 2048, 4096, 8192, 16384, 32768
+DH_FLAG_ACT_H16 = 65536
 MODES = {
     "fp32": 0,                                             # every contraction in fp32 FMA (strict)
     "fp32_tcdec": DH_FLAG_DEC_TC | DH_FLAG_DEC_TC_X3,      # strict + the 3xTF32 (fp32-grade) tensor-core decoder
@@ -57,6 +58,11 @@ MODES = {
     # reduced precision: BF16 operands in every convolution (fp32 storage / accumulation), single-pass FP16 stem (its input is an
     # image), 3xTF32 decoder
     "bf16": DH_FLAG_CONV_TC | DH_FLAG_TC_BF16 | DH_FLAG_TC_STRIDE2 | DH_FLAG_STEM_TC | DH_FLAG_DEC_TC | DH_FLAG_DEC_TC_X3,
+    # reduced precision, half the activation bytes: "f16" operands AND every workspace tensor stored as one FP16 plane (2 bytes
+    # per element, saturating at +-65504; tokenizer partials / token memories / decoder tables stay fp32), single-pass FP16
+    # convolutions (conv_tc3.cu single-plane form), 3xTF32 decoder
+    "h16": DH_FLAG_CONV_TC | DH_FLAG_TC_MAIN_F16 | DH_FLAG_TC_STRIDE2 | DH_FLAG_STEM_TC | DH_FLAG_DEC_TC | DH_FLAG_DEC_TC_X3
+           | DH_FLAG_ACT_H16 | DH_FLAG_PDL,
     "tf32_fast": DH_FLAG_CONV_TC | DH_FLAG_TC_STRIDE2 | DH_FLAG_STEM_TC | DH_FLAG_DEC_TC,   # 1xTF32 decoder too
 }
 

@@ -66,12 +66,18 @@ extern "C" {
                                    * the tokenizer's 1x1 squeeze runs on the tensor cores with the softmax partials in its epilogue */
 #define DH_FLAG_PDL         32768 /* programmatic dependent launch between consecutive launches of a stream (prologues overlap the previous
                                    * launch's tail; every kernel waits with griddepcontrol.wait before touching its inputs) */
+#define DH_FLAG_ACT_H16     65536 /* with CONV_TC | TC_MAIN_F16 | TC_STRIDE2 | STEM_TC | DEC_TC (and none of ACT_SPLIT, TC_3XTF32, TC_BF16,
+                                   * CONV_TC_V1; dahitra_forward returns DH_E_VARIANT otherwise): every tensor the forward writes to its
+                                   * workspace is stored as ONE FP16 plane (round to nearest, saturating at +-65504; 2 bytes per element)
+                                   * except the tokenizer partials, token memories and decoder tables; single-pass FP16 convolutions on
+                                   * conv_tc3.cu's single-plane form, FP16 max pools and classifier input.  Inputs and logits stay fp32 */
 /* the modes dahitra_b200.engine.MODES names (DESIGN.md "Precision modes") */
 #define DH_FLAGS_TF32X3     (DH_FLAG_CONV_TC | DH_FLAG_TC_3XTF32 | DH_FLAG_TC_X3_BF16 | DH_FLAG_TC_MAIN_F16 | DH_FLAG_TC_FOLD | DH_FLAG_TC_STRIDE2 | \
                              DH_FLAG_STEM_TC | DH_FLAG_DEC_TC | DH_FLAG_DEC_TC_X3 | DH_FLAG_ACT_SPLIT | DH_FLAG_PDL)   /* default: every product error-compensated, fp32-grade */
 #define DH_FLAGS_TF32       (DH_FLAG_CONV_TC | DH_FLAG_TC_STRIDE2 | DH_FLAG_STEM_TC | DH_FLAG_DEC_TC | DH_FLAG_DEC_TC_X3)   /* single-pass TF32 convs */
 #define DH_FLAGS_F16        (DH_FLAGS_TF32 | DH_FLAG_TC_MAIN_F16)                    /* single-pass FP16 conv operands */
 #define DH_FLAGS_BF16       (DH_FLAGS_TF32 | DH_FLAG_TC_BF16)                        /* single-pass BF16 conv operands */
+#define DH_FLAGS_H16        (DH_FLAGS_F16 | DH_FLAG_ACT_H16 | DH_FLAG_PDL)           /* FP16 operands AND FP16 activation storage */
 
 /* ---- prepared-weight table -------------------------------------------------------------------
  * dahitra_forward takes `const void* const* weights` with DH_W_COUNT slots, each a device pointer to
@@ -215,7 +221,8 @@ int dahitra_stem(const float* x, long long x_batch_stride, int N, int H, int W,
                  const float* w, const float* bias, float* out, void* stream);
 
 /* Same stem on the tensor cores: x3 = 0 TF32 operands, 1 error-compensated 3xTF32, 2 folded FP16 (fp32-grade for |x| <= 65504; the default mode's stem), 3 single-pass FP16 (the f16 / bf16 modes' stem); wtc = DH_W_STEM_WTC image.
- * x3 | 256 (forms 2 and 3): out receives split16 planes instead of fp32. */
+ * x3 | 256 (forms 2 and 3): out receives split16 planes instead of fp32.
+ * x3 | 512 (form 3 only): out receives one FP16 plane [N][H/2][W/2][64] (the h16 mode). */
 int dahitra_stem_tc(const float* x, long long x_batch_stride, int N, int H, int W,
                     const float* wtc, const float* bias, float* out, int x3, void* stream);
 
@@ -262,7 +269,8 @@ int dahitra_pixel_decoder(const float* x, const float* pos, const float* tables,
 #define DH_DECTC_LAYER_FLOATS  (1024 + 1024 + 32 + 32 + 32 + 2048)
 int dahitra_decoder_tables_tc(const float* mem, int B, int first_call, int ncalls, const float* dec_pack, int heads,
                               int depth, float* tables, void* stream);
-/* x3 | 256: out receives split16 planes instead of fp32 */
+/* x3 | 256: out receives split16 planes instead of fp32.
+ * x3 | 512: x, skip and out are one FP16 plane each (the h16 mode); the arithmetic inside is the same, out = f16(result). */
 int dahitra_pixel_decoder_tc(const float* x, const float* pos, const float* tables, const float* dectc_pack,
                              int nimg, int h, int w, int heads, int depth, const float* skip, int skip_up, int x3,
                              float* out, void* stream);
@@ -274,6 +282,8 @@ int dahitra_split_pack(const float* in, long long n, void* out_split, void* stre
 int dahitra_split_unpack(const void* in_split, long long n, float* out, void* stream);
 /* MaxPool2d(3, 2, 1) on a split16 NHWC tensor (compares reconstructed values; the winner's planes are reproduced exactly) */
 int dahitra_maxpool3x3s2_split(const void* in_split, int N, int H, int W, int C, void* out_split, void* stream);
+/* MaxPool2d(3, 2, 1) on one FP16 NHWC plane (the h16 mode; exact, C % 8 == 0) */
+int dahitra_maxpool3x3s2_h16(const void* in_h16, int N, int H, int W, int C, void* out_h16, void* stream);
 /* Convolution over split16 inputs with all three partial products on FP16 MMAs (file header of conv_tc3.cu):
  *   in0 / in1      split16 NHWC sources (virtual channel concat, C1 may be 0); in*_plane = elements between their hi and lo
  *                  planes (0 = N*inH*inW*C; larger when they are sub-ranges of the images of one tensor)
@@ -285,7 +295,11 @@ int dahitra_maxpool3x3s2_split(const void* in_split, int N, int H, int W, int C,
  *                    nchunk = ceil(inH/16) * ceil(inW/8), w_tok [32][4]  (see dahitra_squeeze_tokens)
  *                  scheduling bits, OR-ed in (results do not depend on them): 16 = single CTAs, 32 = CTA pairs
  *                  (tcgen05 cta_group::2; default: chosen per shape), 64 = stream the filter from L2 even where it
- *                  would fit in shared memory */
+ *                  would fit in shared memory
+ *                  storage bit, OR-ed in: 128 = the h16 mode's format: in0, in1, a split res (res_split = 1) and a split out
+ *                  (out_split = 1, also with the pixel-shuffle store) are ONE FP16 plane each, in*_plane is ignored, and only
+ *                  h_w (plane 3) of the filter is read: one FP16 MMA per (tap, chunk, K step).  With 128 a CTA-pair request
+ *                  (bit 32, or DAHITRA_TC3_CG) returns DH_E_VARIANT */
 int dahitra_conv2d_split(const void* in0, const void* in1, int C0, int C1, long long in0_plane, long long in1_plane,
                          int N, int inH, int inW, int K, int stride, int Cout, const float* wt, const float* bias,
                          const void* res, int res_split, int relu, void* out, int out_split, int mode,
@@ -295,6 +309,10 @@ int dahitra_conv2d_split(const void* in0, const void* in1, int C0, int C1, long 
  * (reference models/networks.py:1249,1355; harness argmax models/evaluator.py:89-92). */
 int dahitra_classifier(const float* in, int N, int H, int W, int nc, const float* w, const float* bias,
                        float* logits, unsigned char* argmax_u8, void* stream);
+/* The same classifier on one FP16 NHWC plane [N][H][W][32] (the h16 mode): TMA halo boxes of FP16, converted to fp32 on the
+ * shared-memory read; fp32 sums, fp32 NCHW logits, uint8 argmax with the lowest-index tie rule. */
+int dahitra_classifier_h16(const void* in_h16, int N, int H, int W, int nc, const float* w, const float* bias,
+                           float* logits, unsigned char* argmax_u8, void* stream);
 
 /* ---- training step (SURVEY.md §8 f4): pixel decoder forward that keeps the layer inputs + its hand-written backward ----------
  * Replaces, on the training route, the per-pixel arithmetic of reference models/help_funcs.py:66-114,170-186 and the
