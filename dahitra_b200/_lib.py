@@ -164,6 +164,10 @@ SIGNATURES = {
     "dahitra_tokenizer_train_chunks": (_I, [_I]),
     "dahitra_tokenizer_train_fwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "dahitra_tokenizer_train_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
+    "dahitra_pixel_decoder_train_fwd_ex": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "dahitra_pixel_decoder_train_bwd_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
+    "dahitra_tokenizer_train_fwd_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "dahitra_tokenizer_train_bwd_ex": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "dahitra_conv2d_split": (_I, [_P, _P, _I, _I, _LL, _LL, _I, _I, _I, _I, _I, _I, _P, _P, _P, _I, _I, _P, _I, _I, _P, _P, _P]),
     "dahitra_maxpool3x3s2_h16": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "dahitra_classifier_h16": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),

@@ -17,7 +17,9 @@
 // LayerNorm parameters, the MLP weights and — through the tokens — the tokenizer, the token encoder and the trunk.
 //
 // Layout: x, out, dx, dout are channel-planar [B][32][N] (= the NCHW tensors of the reference, flattened over h, w): one thread
-// per pixel reads and writes fully coalesced rows, and no transpose to (B, N, 32) is ever made.
+// per pixel reads and writes fully coalesced rows, and no transpose to (B, N, 32) is ever made; or pixel-major [B][N][32]
+// (channels_last).  Their storage type TA is fp32, fp16 or bf16 (train_act.cuh: what autocast hands over); the saved layer
+// inputs xs stay fp32, so the backward recomputes exactly what the forward computed.
 // Table [B][L][DH_TRAIN_TAB_FLOATS(K)]:  A 32K | c0 K | Bv 32K | bo 32 | W1 1024 | b1 32 | W2 1024 | b2 32.
 //
 // Kernel structure: 128 pixels per CTA, one pixel per thread.  Every per-pixel vector that feeds a contraction lives in shared
@@ -30,6 +32,7 @@
 // 1.8x fewer shared-memory wavefronts): correct, but 255 registers with spills and four warps per SM made the backward 40 %
 // SLOWER (0.67 -> 0.86 ms at level 3) — the kernel needs its eight warps per SM to cover the shared-memory latency.
 #include "common.cuh"
+#include "train_act.cuh"
 
 namespace {
 
@@ -148,44 +151,14 @@ __device__ __forceinline__ void softmax4(float (&d)[K]) {
   }
 }
 
-// one pixel's 32 channels from / to a [B][32][N] (planar, PM = false) or [B][N][32] (pixel-major = channels_last, PM = true) tensor
-template <bool PM>
-__device__ __forceinline__ void load_pixel(const float* __restrict__ t, int b, int n, int N, bool live, float (&v)[32]) {
-  if (PM) {
-    const float4* p = reinterpret_cast<const float4*>(t + ((size_t)b * N + n) * 32);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const float4 w = live ? __ldg(p + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-      v[4 * q] = w.x; v[4 * q + 1] = w.y; v[4 * q + 2] = w.z; v[4 * q + 3] = w.w;
-    }
-  } else {
-    const float* p = t + (size_t)b * 32 * N + n;
-#pragma unroll
-    for (int c = 0; c < 32; ++c) v[c] = live ? p[(size_t)c * N] : 0.f;
-  }
-}
-template <bool PM>
-__device__ __forceinline__ void store_pixel(float* __restrict__ t, int b, int n, int N, bool live, const float (&v)[32]) {
-  if (!live) return;
-  if (PM) {
-    float4* p = reinterpret_cast<float4*>(t + ((size_t)b * N + n) * 32);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) p[q] = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-  } else {
-    float* p = t + (size_t)b * 32 * N + n;
-#pragma unroll
-    for (int c = 0; c < 32; ++c) p[(size_t)c * N] = v[c];
-  }
-}
-
 __device__ __forceinline__ void load_table(const float* __restrict__ g, float* __restrict__ s, int T) {
   for (int i = threadIdx.x * 4; i < T; i += PT * 4) *reinterpret_cast<float4*>(s + i) = __ldg(reinterpret_cast<const float4*>(g + i));
 }
 
 // ------------------------------------------------------------------------------------------------ forward (training)
-template <int K, bool PM>
-__global__ void __launch_bounds__(PT) decoder_train_fwd_kernel(const float* __restrict__ x, const float* __restrict__ table,
-                                                               float* __restrict__ xs, float* __restrict__ out, int B, int N, int L) {
+template <int K, bool PM, typename TA>
+__global__ void __launch_bounds__(PT) decoder_train_fwd_kernel(const TA* __restrict__ x, const float* __restrict__ table,
+                                                               float* __restrict__ xs, TA* __restrict__ out, int B, int N, int L) {
   constexpr TabOff O = tab_off(K);
   extern __shared__ __align__(16) float smem[];
   float* tab = smem;                       // O.T floats
@@ -194,11 +167,11 @@ __global__ void __launch_bounds__(PT) decoder_train_fwd_kernel(const float* __re
   const int b = blockIdx.y, tid = threadIdx.x, n = blockIdx.x * PT + tid;
   const bool live = n < N;
   float v[32];
-  load_pixel<PM>(x, b, n, N, live, v);
+  dh_load_pixel<PM>(x, b, n, N, live, v);
   for (int l = 0; l < L; ++l) {
     __syncthreads();                                                   // the previous layer is done with the table
     load_table(table + ((size_t)b * L + l) * O.T, tab, O.T);
-    store_pixel<false>(xs + (size_t)l * B * 32 * N, b, n, N, live, v);  // layer inputs are kept planar (coalesced both ways)
+    dh_store_pixel<false>(xs + (size_t)l * B * 32 * N, b, n, N, live, v);  // layer inputs are kept planar (coalesced both ways)
     {
       float xn[32];
       layer_norm32(v, xn);
@@ -234,7 +207,7 @@ __global__ void __launch_bounds__(PT) decoder_train_fwd_kernel(const float* __re
     for (int c = 0; c < 32; ++c) v[c] += tab[O.b2 + c];
     matvec<32, 32>(bufB + tid, tab + O.W2, v);                         // z = y + b2 + gelu(h) W2
   }
-  store_pixel<PM>(out, b, n, N, live, v);
+  dh_store_pixel<PM>(out, b, n, N, live, v);
 }
 
 // ------------------------------------------------------------------------------------------------ backward
@@ -268,9 +241,9 @@ __device__ __forceinline__ void wgrad(const float* __restrict__ a, const float* 
   }
 }
 
-template <int K, bool PM>
-__global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const float* __restrict__ dout, const float* __restrict__ xs,
-                                                                  const float* __restrict__ table, float* __restrict__ dx,
+template <int K, bool PM, typename TA>
+__global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const TA* __restrict__ dout, const float* __restrict__ xs,
+                                                                  const float* __restrict__ table, TA* __restrict__ dx,
                                                                   float* __restrict__ dtab, int B, int N, int L) {
   constexpr TabOff O = tab_off(K);
   extern __shared__ __align__(16) float smem[];
@@ -284,7 +257,7 @@ __global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const float* _
   const int b = blockIdx.y, tid = threadIdx.x, n = blockIdx.x * PT + tid;
   const bool live = n < N;
   float dz[32];
-  load_pixel<PM>(dout, b, n, N, live, dz);
+  dh_load_pixel<PM>(dout, b, n, N, live, dz);
   for (int l = L - 1; l >= 0; --l) {
     __syncthreads();                                                   // the previous layer's last wgrad / table reads are done
     load_table(table + ((size_t)b * L + l) * O.T, tab, O.T);
@@ -294,7 +267,7 @@ __global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const float* _
     // ---- recompute the layer's forward; keep p, yn, gelu(h), gelu'(h) in shared memory
     {
       float v[32];
-      load_pixel<false>(xl, b, n, N, live, v);
+      dh_load_pixel<false>(xl, b, n, N, live, v);
       {
         float xn[32];
         rstd1 = layer_norm32(v, xn);
@@ -360,7 +333,7 @@ __global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const float* _
     matvec_t<32, K>(dz, tab + O.Bv, s_dz + tid);                       // dp -> s_dz (own column; last read before barrier (2))
     {
       float v[32], xn[32];                                             // xn again (s_yn is free since barrier (4))
-      load_pixel<false>(xl, b, n, N, live, v);
+      dh_load_pixel<false>(xl, b, n, N, live, v);
       layer_norm32(v, xn);
       store_col(s_yn + tid, xn);
     }
@@ -389,26 +362,26 @@ __global__ void __launch_bounds__(PT, 2) decoder_train_bwd_kernel(const float* _
       for (int c = 0; c < 32; ++c) dz[c] += t[c];                      // dx = dy (residual) + LayerNorm backward
     }
   }
-  store_pixel<PM>(dx, b, n, N, live, dz);
+  dh_store_pixel<PM>(dx, b, n, N, live, dz);
 }
 
-template <int K, bool PM>
-int launch_fwd(const float* x, const float* table, float* xs, float* out, int B, int N, int L, cudaStream_t s) {
+template <int K, bool PM, typename TA>
+int launch_fwd(const TA* x, const float* table, float* xs, TA* out, int B, int N, int L, cudaStream_t s) {
   constexpr TabOff O = tab_off(K);
   const size_t smem = (size_t)(O.T + 2 * 32 * PITCH) * sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(decoder_train_fwd_kernel<K, PM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(decoder_train_fwd_kernel<K, PM, TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  decoder_train_fwd_kernel<K, PM><<<dim3(dh_cdiv(N, PT), B), PT, smem, s>>>(x, table, xs, out, B, N, L);
+  decoder_train_fwd_kernel<K, PM, TA><<<dim3(dh_cdiv(N, PT), B), PT, smem, s>>>(x, table, xs, out, B, N, L);
   DH_CHECK_LAUNCH();
   return 0;
 }
-template <int K, bool PM>
-int launch_bwd(const float* dout, const float* xs, const float* table, float* dx, float* dtab, int B, int N, int L, cudaStream_t s) {
+template <int K, bool PM, typename TA>
+int launch_bwd(const TA* dout, const float* xs, const float* table, TA* dx, float* dtab, int B, int N, int L, cudaStream_t s) {
   constexpr TabOff O = tab_off(K);
   const size_t smem = (size_t)(O.T + (4 * 32 + K) * PITCH) * sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(decoder_train_bwd_kernel<K, PM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(decoder_train_bwd_kernel<K, PM, TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  decoder_train_bwd_kernel<K, PM><<<dim3(dh_cdiv(N, PT), B), PT, smem, s>>>(dout, xs, table, dx, dtab, B, N, L);
+  decoder_train_bwd_kernel<K, PM, TA><<<dim3(dh_cdiv(N, PT), B), PT, smem, s>>>(dout, xs, table, dx, dtab, B, N, L);
   DH_CHECK_LAUNCH();
   return 0;
 }
@@ -417,29 +390,57 @@ int launch_bwd(const float* dout, const float* xs, const float* table, float* dx
 
 extern "C" int dahitra_pixel_decoder_train_blocks(int npix) { return npix > 0 ? dh_cdiv(npix, PT) : 0; }
 
-extern "C" int dahitra_pixel_decoder_train_fwd(const float* x, const float* tables, float* xs, float* out, int nimg, int npix,
-                                               int heads, int depth, int pixel_major, void* stream) {
+extern "C" int dahitra_pixel_decoder_train_fwd_ex(const void* x, const float* tables, float* xs, void* out, int nimg, int npix,
+                                                  int heads, int depth, int pixel_major, int act_dtype, void* stream) {
+  const int eb = dh_act_bytes(act_dtype);
+  DH_REQUIRE(eb > 0, DH_E_VARIANT);
   DH_REQUIRE(x && tables && xs && out, DH_E_NULL);
   DH_REQUIRE(nimg > 0 && npix > 0 && depth > 0 && nimg <= 65535, DH_E_SHAPE);
   DH_REQUIRE(heads == 4 || heads == 8, DH_E_SHAPE);
-  DH_REQUIRE(dh_aligned16(tables) && (!pixel_major || (dh_aligned16(x) && dh_aligned16(out))), DH_E_ALIGN);
+  const int xal = pixel_major ? 16 : eb;
+  DH_REQUIRE(dh_aligned16(tables) && dh_aligned(x, xal) && dh_aligned(out, xal), DH_E_ALIGN);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (pixel_major)
-    return heads == 4 ? launch_fwd<16, true>(x, tables, xs, out, nimg, npix, depth, s) : launch_fwd<32, true>(x, tables, xs, out, nimg, npix, depth, s);
-  return heads == 4 ? launch_fwd<16, false>(x, tables, xs, out, nimg, npix, depth, s) : launch_fwd<32, false>(x, tables, xs, out, nimg, npix, depth, s);
+  return dh_act_dispatch(act_dtype, [&](auto t) {
+    using TA = decltype(t);
+    const TA* xa = static_cast<const TA*>(x);
+    TA* oa = static_cast<TA*>(out);
+    if (pixel_major)
+      return heads == 4 ? launch_fwd<16, true>(xa, tables, xs, oa, nimg, npix, depth, s) : launch_fwd<32, true>(xa, tables, xs, oa, nimg, npix, depth, s);
+    return heads == 4 ? launch_fwd<16, false>(xa, tables, xs, oa, nimg, npix, depth, s) : launch_fwd<32, false>(xa, tables, xs, oa, nimg, npix, depth, s);
+  });
+}
+
+extern "C" int dahitra_pixel_decoder_train_bwd_ex(const void* dout, const float* xs, const float* tables, void* dx,
+                                                  float* dtables_partial, int nimg, int npix, int heads, int depth, int pixel_major,
+                                                  int act_dtype, void* stream) {
+  const int eb = dh_act_bytes(act_dtype);
+  DH_REQUIRE(eb > 0, DH_E_VARIANT);
+  DH_REQUIRE(dout && xs && tables && dx && dtables_partial, DH_E_NULL);
+  DH_REQUIRE(nimg > 0 && npix > 0 && depth > 0 && nimg <= 65535, DH_E_SHAPE);
+  DH_REQUIRE(heads == 4 || heads == 8, DH_E_SHAPE);
+  const int xal = pixel_major ? 16 : eb;
+  DH_REQUIRE(dh_aligned16(tables) && dh_aligned(dout, xal) && dh_aligned(dx, xal), DH_E_ALIGN);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  return dh_act_dispatch(act_dtype, [&](auto t) {
+    using TA = decltype(t);
+    const TA* da = static_cast<const TA*>(dout);
+    TA* xa = static_cast<TA*>(dx);
+    if (pixel_major)
+      return heads == 4 ? launch_bwd<16, true>(da, xs, tables, xa, dtables_partial, nimg, npix, depth, s)
+                        : launch_bwd<32, true>(da, xs, tables, xa, dtables_partial, nimg, npix, depth, s);
+    return heads == 4 ? launch_bwd<16, false>(da, xs, tables, xa, dtables_partial, nimg, npix, depth, s)
+                      : launch_bwd<32, false>(da, xs, tables, xa, dtables_partial, nimg, npix, depth, s);
+  });
+}
+
+extern "C" int dahitra_pixel_decoder_train_fwd(const float* x, const float* tables, float* xs, float* out, int nimg, int npix,
+                                               int heads, int depth, int pixel_major, void* stream) {
+  return dahitra_pixel_decoder_train_fwd_ex(x, tables, xs, out, nimg, npix, heads, depth, pixel_major, DH_ACT_F32, stream);
 }
 
 extern "C" int dahitra_pixel_decoder_train_bwd(const float* dout, const float* xs, const float* tables, float* dx,
                                                float* dtables_partial, int nimg, int npix, int heads, int depth, int pixel_major,
                                                void* stream) {
-  DH_REQUIRE(dout && xs && tables && dx && dtables_partial, DH_E_NULL);
-  DH_REQUIRE(nimg > 0 && npix > 0 && depth > 0 && nimg <= 65535, DH_E_SHAPE);
-  DH_REQUIRE(heads == 4 || heads == 8, DH_E_SHAPE);
-  DH_REQUIRE(dh_aligned16(tables) && (!pixel_major || (dh_aligned16(dout) && dh_aligned16(dx))), DH_E_ALIGN);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  if (pixel_major)
-    return heads == 4 ? launch_bwd<16, true>(dout, xs, tables, dx, dtables_partial, nimg, npix, depth, s)
-                      : launch_bwd<32, true>(dout, xs, tables, dx, dtables_partial, nimg, npix, depth, s);
-  return heads == 4 ? launch_bwd<16, false>(dout, xs, tables, dx, dtables_partial, nimg, npix, depth, s)
-                    : launch_bwd<32, false>(dout, xs, tables, dx, dtables_partial, nimg, npix, depth, s);
+  return dahitra_pixel_decoder_train_bwd_ex(dout, xs, tables, dx, dtables_partial, nimg, npix, heads, depth, pixel_major,
+                                            DH_ACT_F32, stream);
 }

@@ -6,31 +6,17 @@
 // normalisation term collapses onto the tokens:  sum_n p[l][n] dp[l][n] = sum_c dtok[l][c] tok[l][c]:
 //     dp[l][n] = sum_c dtok[l][c] x[c][n]            da[l][n] = p[l][n] (dp[l][n] - sum_c dtok[l][c] tok[l][c])
 //     dx[c][n] = sum_l p[l][n] dtok[l][c] + Wt[l][c] da[l][n]          dWt[l][c] = sum_{b, n} da[l][n] x[c][n]
-// Layouts: x / dx channel-planar [B][32][N] (NCHW) or pixel-major [B][N][32] (channels_last), as in train_decoder.cu.
+// Layouts: x / dx channel-planar [B][32][N] (NCHW) or pixel-major [B][N][32] (channels_last), stored as fp32, fp16 or bf16
+// (train_act.cuh), as in train_decoder.cu; tokens, stats, Wt and every partial are fp32.
 // One pixel per thread, 256 pixels per CTA; per-CTA partial sums are written (never accumulated atomically) and reduced by a
 // second tiny kernel (forward) or by the caller (dWt): deterministic.
 #include "common.cuh"
+#include "train_act.cuh"
 
 namespace {
 
 constexpr int TT = 256;          // pixels (= threads) per CTA
 constexpr int TP = TT + 4;       // row pitch of the staged [component][pixel] arrays
-
-template <bool PM>
-__device__ __forceinline__ void tk_load(const float* __restrict__ t, int b, int n, int N, bool live, float (&v)[32]) {
-  if (PM) {
-    const float4* p = reinterpret_cast<const float4*>(t + ((size_t)b * N + n) * 32);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const float4 w = live ? __ldg(p + q) : make_float4(0.f, 0.f, 0.f, 0.f);
-      v[4 * q] = w.x; v[4 * q + 1] = w.y; v[4 * q + 2] = w.z; v[4 * q + 3] = w.w;
-    }
-  } else {
-    const float* p = t + (size_t)b * 32 * N + n;
-#pragma unroll
-    for (int c = 0; c < 32; ++c) v[c] = live ? p[(size_t)c * N] : 0.f;
-  }
-}
 
 __device__ __forceinline__ float block_max(float v, float* red) {   // red: >= 8 floats; all threads get the result
   v = warp_max(v);
@@ -44,8 +30,8 @@ __device__ __forceinline__ float block_max(float v, float* red) {   // red: >= 8
 }
 
 // per 256-pixel chunk: m[l] = max a, s[l] = sum exp(a - m), t[l][c] = sum exp(a - m) x[c]   -> part[b][chunk][l][34]
-template <bool PM>
-__global__ void __launch_bounds__(TT) tok_fwd_partial_kernel(const float* __restrict__ x, const float* __restrict__ wt,
+template <bool PM, typename TA>
+__global__ void __launch_bounds__(TT) tok_fwd_partial_kernel(const TA* __restrict__ x, const float* __restrict__ wt,
                                                              float* __restrict__ part, int N) {
   __shared__ __align__(16) float s_x[32 * TP];
   __shared__ __align__(16) float s_e[4 * TP];
@@ -54,7 +40,7 @@ __global__ void __launch_bounds__(TT) tok_fwd_partial_kernel(const float* __rest
   const bool live = n < N;
   if (tid < 128) s_w[tid] = wt[tid];
   float v[32];
-  tk_load<PM>(x, b, n, N, live, v);
+  dh_load_pixel<PM>(x, b, n, N, live, v);
 #pragma unroll
   for (int c = 0; c < 32; ++c) s_x[c * TP + tid] = v[c];
   __syncthreads();
@@ -108,10 +94,10 @@ __global__ void __launch_bounds__(128) tok_merge_kernel(const float* __restrict_
   if (c == 0) { stats[(b * 4 + l) * 2] = M; stats[(b * 4 + l) * 2 + 1] = Z; }
 }
 
-template <bool PM>
-__global__ void __launch_bounds__(TT) tok_bwd_kernel(const float* __restrict__ x, const float* __restrict__ wt,
+template <bool PM, typename TA>
+__global__ void __launch_bounds__(TT) tok_bwd_kernel(const TA* __restrict__ x, const float* __restrict__ wt,
                                                      const float* __restrict__ tok, const float* __restrict__ stats,
-                                                     const float* __restrict__ dtok, float* __restrict__ dx,
+                                                     const float* __restrict__ dtok, TA* __restrict__ dx,
                                                      float* __restrict__ dwt_part, int N) {
   __shared__ __align__(16) float s_x[32 * TP];
   __shared__ __align__(16) float s_da[4 * TP];
@@ -126,7 +112,7 @@ __global__ void __launch_bounds__(TT) tok_bwd_kernel(const float* __restrict__ x
     if ((tid & 31) == 0) s_s[tid >> 5] = s;
   }
   float v[32];
-  tk_load<PM>(x, b, n, N, live, v);
+  dh_load_pixel<PM>(x, b, n, N, live, v);
 #pragma unroll
   for (int c = 0; c < 32; ++c) s_x[c * TP + tid] = v[c];
   __syncthreads();
@@ -149,15 +135,7 @@ __global__ void __launch_bounds__(TT) tok_bwd_kernel(const float* __restrict__ x
       for (int l = 0; l < 4; ++l) acc = fmaf(p[l], s_dt[l * 32 + c], fmaf(s_w[l * 32 + c], da[l], acc));
       g[c] = acc;
     }
-    if (PM) {
-      float4* o = reinterpret_cast<float4*>(dx + ((size_t)b * N + n) * 32);
-#pragma unroll
-      for (int q = 0; q < 8; ++q) o[q] = make_float4(g[4 * q], g[4 * q + 1], g[4 * q + 2], g[4 * q + 3]);
-    } else {
-      float* o = dx + (size_t)b * 32 * N + n;
-#pragma unroll
-      for (int c = 0; c < 32; ++c) o[(size_t)c * N] = g[c];
-    }
+    dh_store_pixel<PM>(dx, b, n, N, true, g);
   }
   __syncthreads();
   if (tid < 128) {                                   // dWt partial of this chunk: thread (l, c)
@@ -178,31 +156,57 @@ __global__ void __launch_bounds__(TT) tok_bwd_kernel(const float* __restrict__ x
 
 extern "C" int dahitra_tokenizer_train_chunks(int npix) { return npix > 0 ? dh_cdiv(npix, TT) : 0; }
 
-extern "C" int dahitra_tokenizer_train_fwd(const float* x, const float* w_tok, float* partials, float* tokens, float* stats,
-                                           int nimg, int npix, int pixel_major, void* stream) {
+extern "C" int dahitra_tokenizer_train_fwd_ex(const void* x, const float* w_tok, float* partials, float* tokens, float* stats,
+                                              int nimg, int npix, int pixel_major, int act_dtype, void* stream) {
+  const int eb = dh_act_bytes(act_dtype);
+  DH_REQUIRE(eb > 0, DH_E_VARIANT);
   DH_REQUIRE(x && w_tok && partials && tokens && stats, DH_E_NULL);
   DH_REQUIRE(nimg > 0 && npix > 0 && nimg <= 65535, DH_E_SHAPE);
-  DH_REQUIRE(!pixel_major || dh_aligned16(x), DH_E_ALIGN);
+  DH_REQUIRE(dh_aligned(x, pixel_major ? 16 : eb), DH_E_ALIGN);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const dim3 grid(dh_cdiv(npix, TT), nimg);
-  if (pixel_major) tok_fwd_partial_kernel<true><<<grid, TT, 0, s>>>(x, w_tok, partials, npix);
-  else tok_fwd_partial_kernel<false><<<grid, TT, 0, s>>>(x, w_tok, partials, npix);
+  dh_act_dispatch(act_dtype, [&](auto t) {
+    using TA = decltype(t);
+    if (pixel_major) tok_fwd_partial_kernel<true, TA><<<grid, TT, 0, s>>>(static_cast<const TA*>(x), w_tok, partials, npix);
+    else tok_fwd_partial_kernel<false, TA><<<grid, TT, 0, s>>>(static_cast<const TA*>(x), w_tok, partials, npix);
+    return 0;
+  });
   DH_CHECK_LAUNCH();
   tok_merge_kernel<<<nimg, 128, 0, s>>>(partials, (int)grid.x, tokens, stats);
   DH_CHECK_LAUNCH();
   return 0;
 }
 
+extern "C" int dahitra_tokenizer_train_bwd_ex(const void* x, const float* w_tok, const float* tokens, const float* stats,
+                                              const float* dtokens, void* dx, float* dw_partial, int nimg, int npix,
+                                              int pixel_major, int act_dtype, void* stream) {
+  const int eb = dh_act_bytes(act_dtype);
+  DH_REQUIRE(eb > 0, DH_E_VARIANT);
+  DH_REQUIRE(x && w_tok && tokens && stats && dtokens && dx && dw_partial, DH_E_NULL);
+  DH_REQUIRE(nimg > 0 && npix > 0 && nimg <= 65535, DH_E_SHAPE);
+  DH_REQUIRE(dh_aligned(x, pixel_major ? 16 : eb) && dh_aligned(dx, pixel_major ? 16 : eb), DH_E_ALIGN);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const dim3 grid(dh_cdiv(npix, TT), nimg);
+  dh_act_dispatch(act_dtype, [&](auto t) {
+    using TA = decltype(t);
+    const TA* xa = static_cast<const TA*>(x);
+    TA* da = static_cast<TA*>(dx);
+    if (pixel_major) tok_bwd_kernel<true, TA><<<grid, TT, 0, s>>>(xa, w_tok, tokens, stats, dtokens, da, dw_partial, npix);
+    else tok_bwd_kernel<false, TA><<<grid, TT, 0, s>>>(xa, w_tok, tokens, stats, dtokens, da, dw_partial, npix);
+    return 0;
+  });
+  DH_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int dahitra_tokenizer_train_fwd(const float* x, const float* w_tok, float* partials, float* tokens, float* stats,
+                                           int nimg, int npix, int pixel_major, void* stream) {
+  return dahitra_tokenizer_train_fwd_ex(x, w_tok, partials, tokens, stats, nimg, npix, pixel_major, DH_ACT_F32, stream);
+}
+
 extern "C" int dahitra_tokenizer_train_bwd(const float* x, const float* w_tok, const float* tokens, const float* stats,
                                            const float* dtokens, float* dx, float* dw_partial, int nimg, int npix,
                                            int pixel_major, void* stream) {
-  DH_REQUIRE(x && w_tok && tokens && stats && dtokens && dx && dw_partial, DH_E_NULL);
-  DH_REQUIRE(nimg > 0 && npix > 0 && nimg <= 65535, DH_E_SHAPE);
-  DH_REQUIRE(!pixel_major || (dh_aligned16(x) && dh_aligned16(dx)), DH_E_ALIGN);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const dim3 grid(dh_cdiv(npix, TT), nimg);
-  if (pixel_major) tok_bwd_kernel<true><<<grid, TT, 0, s>>>(x, w_tok, tokens, stats, dtokens, dx, dw_partial, npix);
-  else tok_bwd_kernel<false><<<grid, TT, 0, s>>>(x, w_tok, tokens, stats, dtokens, dx, dw_partial, npix);
-  DH_CHECK_LAUNCH();
-  return 0;
+  return dahitra_tokenizer_train_bwd_ex(x, w_tok, tokens, stats, dtokens, dx, dw_partial, nimg, npix, pixel_major, DH_ACT_F32,
+                                        stream);
 }

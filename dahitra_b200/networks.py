@@ -241,11 +241,13 @@ class BASE_Transformer_UNet(nn.Module):
             nb = f1.shape[0]
             x12 = sq(torch.cat([f1, f2]) if f12 is None else f12)
             t12 = T.semantic_tokens(x12, tk.weight)
-            tok = torch.cat([t12[:nb], t12[nb:]], dim=1)
-            if self.with_pos:
-                tok = tok + getattr(self, f"pos_embedding_{k}")
-            t1, t2 = enc(tok).chunk(2, dim=1)
-            tab = dec.train_tables(torch.cat([t1, t2, (t2 - t1).abs()]))
+            # tokens, token encoder and tables are a few KB: fp32 even under autocast (16 bits would only cost accuracy)
+            with torch.autocast("cuda", enabled=False):
+                tok = torch.cat([t12[:nb], t12[nb:]], dim=1)
+                if self.with_pos:
+                    tok = tok + getattr(self, f"pos_embedding_{k}")
+                t1, t2 = enc(tok).chunk(2, dim=1)
+                tab = dec.train_tables(torch.cat([t1, t2, (t2 - t1).abs()]))
             y12 = decode_native(x12, tab[:2 * nb])
             return decode_native(conv_decode(torch.cat([y12[:nb], y12[nb:]], dim=1)), tab[2 * nb:])
         x1, x2 = sq(f1), sq(f2)

@@ -16,11 +16,21 @@ the module, like the reference's, owns 48 parameters no forward ever reads — a
 
 ``use_graph=False`` runs the same step eagerly (same flat buffer, same all-reduce) — what the CPU / gloo tests exercise.
 The module is generic: any ``nn.Module``, any loss callable, any batch tuple whose last element is the target.
+
+Mixed precision (``amp=torch.float16`` or ``torch.bfloat16``): graph 1 runs the forward and the loss under autocast.  For fp16 the
+step is ``torch.amp.GradScaler`` with its defaults, kept on the device so that nothing waits for the host: graph 1 runs the
+backward from ``loss * scale``; after the all-reduce (so every rank sees the same overflow) graph 2 unscales the flat buffer and
+sets ``found_inf`` (``torch._amp_foreach_non_finite_check_and_unscale_``), the optimizer skips its update on the device when
+``found_inf`` is set (``_step_supports_amp_scaling``: fused Adam, AdamW or SGD), and ``torch._amp_update_scale_`` moves the
+scale.  bf16 has fp32's exponent range and needs no scaler.
 """
 from __future__ import annotations
 
 import torch
 import torch.distributed as dist
+
+# torch.amp.GradScaler's defaults
+INIT_SCALE, GROWTH_FACTOR, BACKOFF_FACTOR, GROWTH_INTERVAL = 2.0 ** 16, 2.0, 0.5, 2000
 
 
 def _grad_view(flat, offset, p):
@@ -45,14 +55,24 @@ class GraphedTrainStep:
                    supported — the state is created by one throw-away step before capture and zeroed again
     group          torch.distributed process group (default: the world group if initialised, else single process);
                    distributed=False keeps the step local even inside an initialised process group
+    amp            None (fp32), torch.float16 (autocast + device-side loss scaling: the optimizer must support
+                   ``_step_supports_amp_scaling``, i.e. fused=True Adam / AdamW / SGD) or torch.bfloat16 (autocast)
     """
 
-    def __init__(self, net, loss_fn, example_batch, make_optimizer, group=None, use_graph=True, warmup=3, distributed=True):
+    def __init__(self, net, loss_fn, example_batch, make_optimizer, group=None, use_graph=True, warmup=3, distributed=True,
+                 amp=None):
+        if amp not in (None, torch.float16, torch.bfloat16):
+            raise ValueError(f"GraphedTrainStep: amp must be None, torch.float16 or torch.bfloat16, not {amp}")
+        self.amp, self.scaled = amp, amp == torch.float16
         self.net, self.loss_fn, self.group = net.train(), loss_fn, group
         self.world = dist.get_world_size(group) if (distributed and dist.is_available() and dist.is_initialized()) else 1
         self.static = [t.clone() for t in example_batch]
         dev = self.static[0].device
         self.use_graph = bool(use_graph) and dev.type == "cuda"
+        if self.scaled:                                                          # GradScaler's state, on the device
+            self.scale = torch.full((1,), INIT_SCALE, dtype=torch.float32, device=dev)
+            self.growth_tracker = torch.zeros(1, dtype=torch.int32, device=dev)
+            self.found_inf = torch.zeros((), dtype=torch.float32, device=dev)
         buffers = [(b, b.clone()) for b in net.buffers()]                       # BatchNorm running stats must not see the warm-up
         for p in net.parameters():
             p.grad = None
@@ -72,8 +92,21 @@ class GraphedTrainStep:
             for p in self.frozen:
                 p.requires_grad_(False)
             self.opt = make_optimizer(self.live)
+            if self.scaled and not getattr(self.opt, "_step_supports_amp_scaling", False):
+                for p in net.parameters():
+                    p.grad = None
+                for p in self.frozen:
+                    p.requires_grad_(True)
+                with torch.no_grad():
+                    for b, s in buffers:
+                        b.copy_(s)
+                raise ValueError(f"GraphedTrainStep(amp=torch.float16): {type(self.opt).__name__} cannot skip a step on the device "
+                                 "when a gradient overflowed, so every step would wait for the host; use an optimizer with "
+                                 "_step_supports_amp_scaling (fused=True Adam, AdamW or SGD)")
+            if self.scaled:
+                self.opt.found_inf = self.found_inf                              # read by the fused step: skip when set
             saved = [p.detach().clone() for p in self.live]
-            self.opt.step()                                                      # creates the optimizer state outside any capture
+            self._optimizer_step()                                               # creates the optimizer state outside any capture
             with torch.no_grad():
                 for p, s in zip(self.live, saved):
                     p.copy_(s)
@@ -83,6 +116,9 @@ class GraphedTrainStep:
                             v.zero_()
                 for b, s in buffers:
                     b.copy_(s)
+                if self.scaled:
+                    self.scale.fill_(INIT_SCALE)
+                    self.growth_tracker.zero_()
             if self.use_graph:
                 self._forward_backward(zero=True)                                # once more with the flat views in place
                 with torch.no_grad():
@@ -97,18 +133,52 @@ class GraphedTrainStep:
             with torch.cuda.graph(self.g_fb):
                 self.loss = self._forward_backward(zero=True)
             with torch.cuda.graph(self.g_opt):
-                self.opt.step()
+                self._optimizer_step()
 
     def _forward_backward(self, zero):
-        loss = self.loss_fn(self.net(*self.static[:-1]), self.static[-1])
+        # graphs need the autocast weight cache off; it changes no value
+        with torch.autocast(self.static[0].device.type, dtype=self.amp, cache_enabled=False) if self.amp else _null():
+            loss = self.loss_fn(self.net(*self.static[:-1]), self.static[-1])
         if not zero:                                                             # warm-up: marks the live parameters
             loss.backward()
             return loss.detach()
         # the gradients are WRITTEN into the flat buffer (no zeroing pass, no per-parameter accumulation kernels): autograd
         # returns them, one multi-tensor copy moves them into the views the optimizer reads as .grad
-        grads = torch.autograd.grad(loss, self.live)
+        grads = torch.autograd.grad(loss * self.scale if self.scaled else loss, self.live)
         torch._foreach_copy_([p.grad for p in self.live], list(grads))
         return loss.detach()
+
+    def _optimizer_step(self):
+        if self.scaled:                                                          # GradScaler.unscale_ / step / update
+            self.found_inf.zero_()
+            torch._amp_foreach_non_finite_check_and_unscale_([self.flat], self.found_inf, self.scale.double().reciprocal().float())
+        self.opt.step()
+        if self.scaled:
+            torch._amp_update_scale_(self.scale, self.growth_tracker, self.found_inf, GROWTH_FACTOR, BACKOFF_FACTOR, GROWTH_INTERVAL)
+
+    def scaler_state_dict(self):
+        """the loss scaler's state in torch.amp.GradScaler.state_dict() form ({} without one, like a disabled GradScaler), so a
+        checkpoint moves between this step and an eager GradScaler loop"""
+        if not self.scaled:
+            return {}
+        return {"scale": float(self.scale), "growth_factor": GROWTH_FACTOR, "backoff_factor": BACKOFF_FACTOR,
+                "growth_interval": GROWTH_INTERVAL, "_growth_tracker": int(self.growth_tracker)}
+
+    def load_scaler_state_dict(self, state):
+        """restore a torch.amp.GradScaler.state_dict() (or scaler_state_dict()); the growth / backoff settings are baked into the
+        captured step and must be GradScaler's defaults"""
+        if not self.scaled:
+            if state:
+                raise ValueError("GraphedTrainStep.load_scaler_state_dict: this step has no loss scaler (amp is not torch.float16)")
+            return
+        if not state:
+            raise ValueError("GraphedTrainStep.load_scaler_state_dict: the state is empty (saved from a disabled GradScaler?)")
+        fixed = {"growth_factor": GROWTH_FACTOR, "backoff_factor": BACKOFF_FACTOR, "growth_interval": GROWTH_INTERVAL}
+        for k, v in fixed.items():
+            if state[k] != v:
+                raise ValueError(f"GraphedTrainStep.load_scaler_state_dict: {k} = {state[k]}, the step runs with {v}")
+        self.scale.fill_(state["scale"])
+        self.growth_tracker.fill_(state["_growth_tracker"])
 
     def all_reduce(self):
         if self.world > 1:
@@ -136,7 +206,7 @@ class GraphedTrainStep:
         if self.use_graph:
             self.g_opt.replay()
         else:
-            self.opt.step()
+            self._optimizer_step()
         return self.loss
 
 

@@ -12,9 +12,15 @@ module's autograd route.  What that route spends its device time on is the pixel
   differentiable torch ops on tensors of a few KB, so autograd carries the table gradients on to Wq / Wk / Wv / Wo, the
   LayerNorm affines, the MLP, the tokens and everything upstream of the tokens).
 
+Mixed precision: both accept x in fp32, fp16 or bf16 (what autocast hands them) and keep x's dtype for the activations that
+leave them (the decoder's output, every dL/dx); the kernels convert on load and store and compute in fp32.  Tables, tokens and
+w_tok are fp32 (converted at the boundary, so their gradients flow back through the conversion).
+
 There is no fallback: the functions raise if the CUDA library is missing or the tensors are not on a GPU.
 """
 from __future__ import annotations
+
+import contextlib
 
 import torch
 
@@ -24,6 +30,15 @@ from . import _lib
 def train_tab_floats(heads: int) -> int:
     """DH_TRAIN_TAB_FLOATS of include/dahitra_b200.h"""
     return 65 * 4 * heads + 96 + 2048
+
+
+_ACT = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}         # DH_ACT_* of include/dahitra_b200.h
+
+
+def _act(x):
+    if x.dtype not in _ACT:
+        raise RuntimeError(f"dahitra_b200.training: activations must be fp32, fp16 or bf16, got {x.dtype}")
+    return _ACT[x.dtype]
 
 
 def _layout(t):
@@ -39,8 +54,9 @@ class _PixelDecoderTrain(torch.autograd.Function):
     def forward(ctx, x, tables, heads):
         if not (x.is_cuda and tables.is_cuda):
             raise RuntimeError("dahitra_b200.training: tensors must be on a CUDA device — there is no CPU path")
-        if x.dtype != torch.float32 or tables.dtype != torch.float32:
-            raise RuntimeError("dahitra_b200.training: fp32 tensors only")
+        act = _act(x)
+        if tables.dtype != torch.float32:
+            raise RuntimeError("dahitra_b200.training: the decoder tables must be fp32")
         B, C = x.shape[:2]
         N = x[0, 0].numel()
         depth = tables.shape[1]
@@ -52,11 +68,11 @@ class _PixelDecoderTrain(torch.autograd.Function):
         xs = torch.empty((depth, B, 32, N), dtype=torch.float32, device=x.device)
         out = torch.empty_like(x)                           # same memory format as x
         with torch.cuda.device(x.device):
-            rc = lib.dahitra_pixel_decoder_train_fwd(x.data_ptr(), tables.data_ptr(), xs.data_ptr(), out.data_ptr(), B, N, heads,
-                                                     depth, pm, torch.cuda.current_stream(x.device).cuda_stream)
-        _lib.check(rc, "dahitra_pixel_decoder_train_fwd")
+            rc = lib.dahitra_pixel_decoder_train_fwd_ex(x.data_ptr(), tables.data_ptr(), xs.data_ptr(), out.data_ptr(), B, N, heads,
+                                                        depth, pm, act, torch.cuda.current_stream(x.device).cuda_stream)
+        _lib.check(rc, "dahitra_pixel_decoder_train_fwd_ex")
         ctx.save_for_backward(xs, tables)
-        ctx.heads = heads
+        ctx.heads, ctx.dtype = heads, x.dtype
         return out
 
     @staticmethod
@@ -65,23 +81,23 @@ class _PixelDecoderTrain(torch.autograd.Function):
         xs, tables = ctx.saved_tensors
         depth, B, _, N = xs.shape
         lib = _lib.load()
-        dout, pm = _layout(dout)
+        dout, pm = _layout(dout.to(ctx.dtype))
         nblk = lib.dahitra_pixel_decoder_train_blocks(N)
         dx = torch.empty_like(dout)
         partial = torch.empty((B, nblk, depth, tables.shape[2]), dtype=torch.float32, device=dout.device)
         with torch.cuda.device(dout.device):
-            rc = lib.dahitra_pixel_decoder_train_bwd(dout.data_ptr(), xs.data_ptr(), tables.data_ptr(), dx.data_ptr(),
-                                                     partial.data_ptr(), B, N, ctx.heads, depth, pm,
-                                                     torch.cuda.current_stream(dout.device).cuda_stream)
-        _lib.check(rc, "dahitra_pixel_decoder_train_bwd")
+            rc = lib.dahitra_pixel_decoder_train_bwd_ex(dout.data_ptr(), xs.data_ptr(), tables.data_ptr(), dx.data_ptr(),
+                                                        partial.data_ptr(), B, N, ctx.heads, depth, pm, _ACT[ctx.dtype],
+                                                        torch.cuda.current_stream(dout.device).cuda_stream)
+        _lib.check(rc, "dahitra_pixel_decoder_train_bwd_ex")
         return dx, partial.sum(1), None
 
 
 def pixel_decoder(x: torch.Tensor, tables: torch.Tensor, heads: int) -> torch.Tensor:
-    """x: (B, 32, N) or (B, 32, h, w) fp32 CUDA — NCHW-contiguous (the kernels' channel-planar layout) or, 4-D only, in
-    torch.channels_last memory format (read pixel-major, no copy); tables (B, depth, DH_TRAIN_TAB_FLOATS(heads)).
-    Returns a tensor of x's shape and memory format.  Differentiable in x and tables (first order)."""
-    return _PixelDecoderTrain.apply(x, tables, heads)
+    """x: (B, 32, N) or (B, 32, h, w) fp32 / fp16 / bf16 CUDA — NCHW-contiguous (the kernels' channel-planar layout) or, 4-D
+    only, in torch.channels_last memory format (read pixel-major, no copy); tables (B, depth, DH_TRAIN_TAB_FLOATS(heads)), used
+    in fp32.  Returns a tensor of x's shape, dtype and memory format.  Differentiable in x and tables (first order)."""
+    return _PixelDecoderTrain.apply(x, tables.float(), heads)
 
 
 class _SemanticTokensTrain(torch.autograd.Function):
@@ -89,8 +105,9 @@ class _SemanticTokensTrain(torch.autograd.Function):
     def forward(ctx, x, w_tok):
         if not (x.is_cuda and w_tok.is_cuda):
             raise RuntimeError("dahitra_b200.training: tensors must be on a CUDA device — there is no CPU path")
-        if x.dtype != torch.float32 or w_tok.dtype != torch.float32:
-            raise RuntimeError("dahitra_b200.training: fp32 tensors only")
+        act = _act(x)
+        if w_tok.dtype != torch.float32:
+            raise RuntimeError("dahitra_b200.training: w_tok must be fp32")
         B, C = x.shape[:2]
         N = x[0, 0].numel()
         if C != 32 or w_tok.numel() != 128:
@@ -102,11 +119,11 @@ class _SemanticTokensTrain(torch.autograd.Function):
         tok = torch.empty((B, 4, 32), dtype=torch.float32, device=x.device)
         stats = torch.empty((B, 4, 2), dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            rc = lib.dahitra_tokenizer_train_fwd(x.data_ptr(), w.data_ptr(), part.data_ptr(), tok.data_ptr(), stats.data_ptr(), B, N, pm,
-                                                 torch.cuda.current_stream(x.device).cuda_stream)
-        _lib.check(rc, "dahitra_tokenizer_train_fwd")
+            rc = lib.dahitra_tokenizer_train_fwd_ex(x.data_ptr(), w.data_ptr(), part.data_ptr(), tok.data_ptr(), stats.data_ptr(), B, N,
+                                                    pm, act, torch.cuda.current_stream(x.device).cuda_stream)
+        _lib.check(rc, "dahitra_tokenizer_train_fwd_ex")
         ctx.save_for_backward(x, w, tok, stats)
-        ctx.pm, ctx.w_shape = pm, w_tok.shape
+        ctx.pm, ctx.w_shape, ctx.act = pm, w_tok.shape, act
         return tok
 
     @staticmethod
@@ -116,21 +133,21 @@ class _SemanticTokensTrain(torch.autograd.Function):
         B = x.shape[0]
         N = x[0, 0].numel()
         lib = _lib.load()
-        dtok = dtok.contiguous()
+        dtok = dtok.float().contiguous()
         dx = torch.empty_like(x)
         dwp = torch.empty((B, lib.dahitra_tokenizer_train_chunks(N), 4, 32), dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            rc = lib.dahitra_tokenizer_train_bwd(x.data_ptr(), w.data_ptr(), tok.data_ptr(), stats.data_ptr(), dtok.data_ptr(),
-                                                 dx.data_ptr(), dwp.data_ptr(), B, N, ctx.pm,
-                                                 torch.cuda.current_stream(x.device).cuda_stream)
-        _lib.check(rc, "dahitra_tokenizer_train_bwd")
+            rc = lib.dahitra_tokenizer_train_bwd_ex(x.data_ptr(), w.data_ptr(), tok.data_ptr(), stats.data_ptr(), dtok.data_ptr(),
+                                                    dx.data_ptr(), dwp.data_ptr(), B, N, ctx.pm, ctx.act,
+                                                    torch.cuda.current_stream(x.device).cuda_stream)
+        _lib.check(rc, "dahitra_tokenizer_train_bwd_ex")
         return dx, dwp.sum((0, 1)).reshape(ctx.w_shape)
 
 
 def semantic_tokens(x: torch.Tensor, w_tok: torch.Tensor) -> torch.Tensor:
-    """x: (B, 32, N) or (B, 32, h, w) fp32 CUDA (NCHW-contiguous or channels_last), w_tok: conv_token_k.weight (4, 32, 1, 1)
-    -> tokens (B, 4, 32).  Differentiable in both (first order)."""
-    return _SemanticTokensTrain.apply(x, w_tok)
+    """x: (B, 32, N) or (B, 32, h, w) fp32 / fp16 / bf16 CUDA (NCHW-contiguous or channels_last), w_tok: conv_token_k.weight
+    (4, 32, 1, 1), used in fp32 -> fp32 tokens (B, 4, 32).  Differentiable in both (first order); dL/dx has x's dtype."""
+    return _SemanticTokensTrain.apply(x, w_tok.float())
 
 
 # ------------------------------------------------------------------------------------------------ graphed autograd route
@@ -151,7 +168,9 @@ class GraphedRoute:
     (torch.cuda.make_graphed_callables): the reference trainer (models/trainer.py:247-262) keeps computing its loss, calling
     backward() and stepping its optimizer eagerly, but the ~1200 launches of the network itself are issued by two graph
     replays.  Built on the first training forward of a given input shape when `net.graphed_training` is set (or
-    DAHITRA_GRAPH_TRAINING=1); other shapes (e.g. a last, smaller batch) run the eager route.  The returned logits live in the
+    DAHITRA_GRAPH_TRAINING=1); other shapes (e.g. a last, smaller batch) run the eager route.  The autocast state (on / off and
+    its dtype) is part of what was captured: a capture made under autocast (captured with the autocast weight cache off, which
+    graphs require) is replayed only under the same autocast, an fp32 capture only without it; the other state runs eagerly.  The returned logits live in the
     graph's static output buffer: they are overwritten by the next training forward, like any graphed callable's."""
 
     def __init__(self, net, xs):
@@ -161,7 +180,9 @@ class GraphedRoute:
         buffers = [(b, b.clone()) for b in net.buffers()]             # the warm-up / capture passes must leave no trace
         grads = [(p, p.grad) for p in net.parameters()]
         sample = tuple(x.detach().clone() for x in xs)
-        self.call = torch.cuda.make_graphed_callables(_Route(net), sample, allow_unused_input=True)
+        amp = self.key[-1]
+        with torch.autocast("cuda", dtype=amp[1], cache_enabled=False) if amp[0] else contextlib.nullcontext():
+            self.call = torch.cuda.make_graphed_callables(_Route(net), sample, allow_unused_input=True)
         with torch.no_grad():
             for b, s in buffers:
                 b.copy_(s)
@@ -173,7 +194,8 @@ class GraphedRoute:
         # input signature + the route switches that were captured (changing one of them afterwards falls back to the eager route)
         flags = tuple(bool(getattr(net, f, True)) for f in ("native_training", "channels_last_training", "paired_trunk_training",
                                                             "collapsed_training"))
-        return tuple((tuple(x.shape), x.dtype, x.device) for x in xs) + (flags,)
+        amp = torch.is_autocast_enabled("cuda")
+        return tuple((tuple(x.shape), x.dtype, x.device) for x in xs) + (flags, (amp, torch.get_autocast_dtype("cuda") if amp else None))
 
     def matches(self, net, xs):
         return self.key == self._key(net, xs) and not any(x.requires_grad for x in xs)

@@ -10,6 +10,8 @@ Mirrors ``BASE_Transformer_UNet`` of reference xBD_code/zoo/model_transformer_en
 """
 from __future__ import annotations
 
+import contextlib
+
 import torch
 from torch import nn
 import torch.nn.functional as F
@@ -115,14 +117,17 @@ class BASE_Transformer_UNet(_LevirNet):
         else:
             x1, x2 = sq(f1), sq(f2)
             tok = torch.cat([tokens(x1), tokens(x2)], dim=1)
-        if self.with_pos and k == 5:
-            tok = tok + self.pos_embedding_3
-        t1, t2 = enc(tok).chunk(2, dim=1)
+        # native route: tokens, token encoder and tables are a few KB, fp32 even under autocast (see networks.py)
+        with torch.autocast("cuda", enabled=False) if native else contextlib.nullcontext():
+            if self.with_pos and k == 5:
+                tok = tok + self.pos_embedding_3
+            t1, t2 = enc(tok).chunk(2, dim=1)
+            tab = dec.train_tables((t2 - t1).abs()) if native else None
         dx = getattr(self, f"conv_decode_{k}")(torch.cat([x1, x2], dim=1))
         if self.with_decoder_pos == 'learned' and k == 5:
             dx = dx + self.pos_embedding_decoder_3
         b, c, h, w = dx.shape
         if native:
-            return T.pixel_decoder(dx, dec.train_tables((t2 - t1).abs()), dec.heads)
+            return T.pixel_decoder(dx, tab, dec.heads)
         run = dec.forward_collapsed if getattr(self, "collapsed_training", True) else dec
         return run(dx.flatten(2).transpose(1, 2), (t2 - t1).abs()).transpose(1, 2).reshape(b, c, h, w)

@@ -334,6 +334,19 @@ int dahitra_pixel_decoder_train_bwd(const float* dout, const float* xs, const fl
                                     float* dtables_partial, int nimg, int npix, int heads, int depth, int pixel_major,
                                     void* stream);
 
+/* Storage type of the per-pixel activations of the training kernels' _ex entry points (mixed-precision training: what autocast
+ * hands over).  Values are converted to fp32 on load and all arithmetic stays fp32; 16-bit stores round to nearest even.  It
+ * applies to x / out / dout / dx only: tables, xs, tokens, stats, w_tok and every partial stay fp32.  Alignment: pixel_major
+ * tensors 16 bytes, planar ones one element.  An unknown act_dtype returns DH_E_VARIANT. */
+#define DH_ACT_F32  0
+#define DH_ACT_F16  1
+#define DH_ACT_BF16 2
+int dahitra_pixel_decoder_train_fwd_ex(const void* x, const float* tables, float* xs, void* out, int nimg, int npix,
+                                       int heads, int depth, int pixel_major, int act_dtype, void* stream);
+int dahitra_pixel_decoder_train_bwd_ex(const void* dout, const float* xs, const float* tables, void* dx,
+                                       float* dtables_partial, int nimg, int npix, int heads, int depth, int pixel_major,
+                                       int act_dtype, void* stream);
+
 /* Semantic tokenizer of the training step: replaces reference models/networks.py:1273-1280 (_forward_semantic_tokens: 1x1 conv
  * 32 -> 4, softmax over the N pixels, einsum to 4 tokens) and its autograd graph.
  *   x, dx        [nimg][32][npix] (pixel_major = 0) or [nimg][npix][32] (pixel_major = 1): the post-ReLU squeeze output
@@ -346,6 +359,12 @@ int dahitra_tokenizer_train_fwd(const float* x, const float* w_tok, float* parti
 int dahitra_tokenizer_train_bwd(const float* x, const float* w_tok, const float* tokens, const float* stats,
                                 const float* dtokens, float* dx, float* dw_partial, int nimg, int npix, int pixel_major,
                                 void* stream);
+/* the same with x / dx stored as act_dtype (DH_ACT_*) */
+int dahitra_tokenizer_train_fwd_ex(const void* x, const float* w_tok, float* partials, float* tokens, float* stats,
+                                   int nimg, int npix, int pixel_major, int act_dtype, void* stream);
+int dahitra_tokenizer_train_bwd_ex(const void* x, const float* w_tok, const float* tokens, const float* stats,
+                                   const float* dtokens, void* dx, float* dw_partial, int nimg, int npix, int pixel_major,
+                                   int act_dtype, void* stream);
 
 /* ---- next to the hot path (SURVEY.md §8 f1) ------------------------------------------------------------ */
 

@@ -3,6 +3,7 @@ Training runs on the stock-autograd route (DESIGN.md "Training step"); under tor
 DistributedDataParallel (NCCL gradient all-reduce, as BASELINE.json's config 4 describes).  After the last step the
 module is switched to eval() and the NATIVE forward is checked against the autograd route on the updated weights.
    python tools/train_step.py [--steps 10]                                   (1 GPU)
+   python tools/train_step.py --graph --amp fp16                             (mixed precision: autocast, device-side loss scaling)
    python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/train_step.py    (DDP)
 Prints one JSON line from rank 0."""
 import argparse, contextlib, json, os, sys, time
@@ -28,7 +29,11 @@ ap.add_argument("--freeze-unused", action="store_true", help="net.freeze_unused_
 ap.add_argument("--graphed-route", action="store_true", help="eager loop (loss, backward(), optimizer as written) with the network's forward / backward replayed from CUDA graphs (net.graphed_training, training.GraphedRoute)")
 ap.add_argument("--foreach-adamw", action="store_true", help="with --graph: torch's foreach AdamW inside the optimizer graph instead of the fused one")
 ap.add_argument("--graph", action="store_true", help="capture forward + backward + AdamW step in ONE CUDA graph and replay it (1 GPU)")
+ap.add_argument("--amp", choices=("fp16", "bf16"), help="mixed precision: forward and loss under autocast; fp16 with loss scaling "
+                "(torch.amp.GradScaler in the eager loop, GraphedTrainStep(amp=torch.float16) with --graph)")
 a = ap.parse_args()
+amp = {None: None, "fp16": torch.float16, "bf16": torch.bfloat16}[a.amp]
+scaler = torch.amp.GradScaler("cuda", enabled=amp == torch.float16)
 world = int(os.environ.get("WORLD_SIZE", "1"))
 rank = int(os.environ.get("RANK", "0"))
 local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -66,9 +71,11 @@ def one_step(sync=True):
     opt.zero_grad(set_to_none=True)
     ctx = model.no_sync() if (world > 1 and not sync) else contextlib.nullcontext()
     with ctx:
-        loss = F.cross_entropy(model(x1, x2), y, weight=w2, ignore_index=255)   # models/losses.py:9-26
-        loss.backward()
-    opt.step()
+        with torch.autocast("cuda", dtype=amp, enabled=amp is not None):
+            loss = F.cross_entropy(model(x1, x2), y, weight=w2, ignore_index=255)   # models/losses.py:9-26
+        scaler.scale(loss).backward()
+    scaler.step(opt)
+    scaler.update()
     return loss
 
 
@@ -96,7 +103,8 @@ if a.graph:
     # dahitra_b200/train_graph.py
     from dahitra_b200.train_graph import GraphedTrainStep
     ts = GraphedTrainStep(net, lambda out, tgt: F.cross_entropy(out, tgt, weight=w2, ignore_index=255), (x1, x2, y),
-                          lambda ps: torch.optim.AdamW(ps, lr=1e-3, weight_decay=0.01, capturable=True, fused=not a.foreach_adamw))
+                          lambda ps: torch.optim.AdamW(ps, lr=1e-3, weight_decay=0.01, capturable=True, fused=not a.foreach_adamw),
+                          amp=amp)
     flat_grad = ts.flat
 step_ms = timed(a.steps)
 dt = step_ms * a.steps / 1e3
@@ -142,6 +150,8 @@ if rank == 0:
                                    + ((", one flat NCCL all-reduce of the live gradients)" if a.graph else ", DDP/NCCL all-reduce)") if world > 1 else ")"),
                           ddp=(None if (world == 1 or a.graph) else ("unused parameters frozen, find_unused_parameters=False" if a.freeze_unused else "find_unused_parameters=True")),
                           loop=("GraphedTrainStep" if a.graph else "eager loop, network forward / backward replayed from CUDA graphs (graphed_training)" if a.graphed_route else "eager"),
+                          precision=("fp32 (TF32 convolutions: torch's default allow_tf32)" if amp is None else f"autocast {a.amp}"
+                                     + (", loss scaling (GradScaler defaults)" if amp == torch.float16 else "")),
                           trunk="one pass per image set" if a.two_pass_trunk else "both image sets per convolution launch, BatchNorm per set", memory_format="contiguous (NCHW)" if a.nchw else "channels_last (set by the module)", steps=a.steps, step_ms=step_ms, steps_per_s=a.steps / dt, pairs_per_s=a.steps * a.batch * world / dt,
                           pairs_per_s_per_gpu=a.steps * a.batch / dt,
                           step_ms_without_allreduce=nosync_ms, exposed_allreduce_share=(None if nosync_ms is None else max(0.0, 1 - nosync_ms / step_ms)),
